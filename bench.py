@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference          # the reference arithmetic (oracle) on the host cores
+    python bench.py --dump-outputs DIR        # also write the last timed step's outputs, to compare two builds
 
 One "step" = one ``training_step`` of ref:src/model.py:259-281 (G phase + AdamW, D phase on a fresh G
 forward + AdamW; L1 + adversarial losses, perceptual term out of scope) on one synthetic batch:
@@ -164,7 +165,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 3)), max(1, min(args.warmup, 1))
+    steps, warmup = args.steps, max(1, min(args.warmup, 1))
     v, ms, cores = cpu_reference_run(steps, warmup, size=64, modality=args.modality)
     sample = f"full GAN step, batch 1 x 64^3 ({args.modality}), fp32 torch CPU, {steps} timed steps after {warmup} warm-up"
     line = {
@@ -305,6 +306,25 @@ def secondary_configs(dev, skip4=False):
     return out
 
 
+DUMP_SAMPLE = 1 << 22    # parameters written per network by --dump-outputs (16 MB of float32 each)
+
+
+def dump_outputs(out_dir, trainer, g_loss, d_loss):
+    """Write what the last timed step hands its caller as ``out_dir/<name>.npy``: the two losses, and the state of the
+    two networks it updated -- a fixed sample of the parameters (indices drawn by ``numpy.random.default_rng(0)`` from
+    the concatenation of ``parameters()`` in order, ascending) and every buffer (BatchNorm statistics, as float64)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"g_loss": g_loss, "d_loss": d_loss}
+    for name, net in (("gen", trainer.gen), ("discr", trainer.discr)):
+        flat = torch.cat([p.detach().reshape(-1) for p in net.parameters()])
+        idx = np.sort(np.random.default_rng(0).choice(flat.numel(), min(DUMP_SAMPLE, flat.numel()), replace=False))
+        arrays[f"{name}_params_sample"] = flat[torch.from_numpy(idx).to(flat.device)]
+        arrays[f"{name}_buffers"] = torch.cat([b.detach().reshape(-1).double() for b in net.buffers()])
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v.cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -321,7 +341,14 @@ def main():
     ap.add_argument("--e2e-x-dtype", default="bf16", choices=["bf16", "fp32"],
                     help="host dtype of the conditioning input x in the end-to-end loop (bf16: same packed bits, "
                          "half the H2D bytes of x)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the losses and the updated network state of the last one to "
+                         "DIR/<name>.npy (inputs and initial weights are seeded: the same arguments give the same inputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path; it is not available with --impl reference")
     if args.impl == "reference":
         return run_reference(args)
     if args.warmup < 3:
@@ -391,6 +418,8 @@ def main():
     ms_step = ms_total.item() / args.steps
     clocks = sampler.stop() if rank == 0 else None
     value = voxels_per_step / (ms_step * 1e-3)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, trainer, g_loss, d_loss)
 
     # ---------------- end-to-end: host buffers, H2D + D2H inside the timed region ----------------
     e2e = None
