@@ -8,8 +8,8 @@
 //   * 1x1x1 convs (heads, final convs)                                            ref:model.py:19-21,83
 //
 // Geometry: an output tile is TD planes x 16 (h) x 8 (w) voxels. Every plane is one UMMA M=128
-// accumulator of NT fp32 columns in TMEM. For each K chunk (kc = 16 or 32 input channels, one
-// swizzle span per voxel row) the producer loads the *halo* of the tile once per A-tile
+// accumulator of NT fp32 columns in TMEM. For each K chunk (kIgemmKc = 32 input channels, one
+// 64-byte swizzle span per voxel row) the producer loads the *halo* of the tile once per A-tile
 // ((16+KH-1) x (8+KW-1) rows per plane) and the MMA thread addresses each filter tap as a
 // row-shifted view of that halo (start address + row offset, SBO = box-width rows) -- no im2col
 // re-load per tap. The skip concatenation is a second tensor map: chunks [0,n0) come from source 0,
@@ -30,7 +30,8 @@
 namespace ub {
 
 constexpr int kMaxTaps = 64;
-constexpr int kMaxAccSets = 4;   // TMEM accumulator sets of the generic kernel (tiles whose epilogue may be pending)
+constexpr int kIgemmKc = 32;     // input channels per K chunk of the generic kernel (64-byte rows, two K = 16 UMMAs)
+constexpr int kMaxAccSets = 2;   // TMEM accumulator sets of the generic kernel (tiles whose epilogue may be pending)
 constexpr int kMaxATiles = 8;
 constexpr int kMaxNTiles = 16;
 
@@ -58,13 +59,13 @@ struct IgemmNTile {
 struct IgemmParams {
   CUtensorMap tm_src[2];
   CUtensorMap tm_w;
-  int n_chunks_src0, n_chunks_total, kc;
+  int n_chunks_src0, n_chunks_total;
   int n_atiles, bw, bh, n_in_planes, in_stride;
   // chunks_per_group > 0 ("group mode", space-to-depth sources): chunk ch belongs to group
   // g = ch / chunks_per_group (the input parity class); the stage holds ONE tile whose origin offset
   // is atile_off[g] and the taps of that chunk are taps[g * ntaps + tp]. The source is parity-planar
   // ([N * groups][D][H][W][chunks_per_group * kc]): channel coordinate (ch % chunks_per_group) * kc,
-  // batch coordinate nb * groups + g. The weight K coordinate is (ch % chunks_per_group) * kc.
+  // batch coordinate nb * groups + g. The weight K coordinate is (ch % chunks_per_group) * kc (kc = kIgemmKc).
   int chunks_per_group;
   int atile_off[kMaxATiles][3];  // (w, h, d) added to in_stride * tile origin
   int ntaps;
@@ -95,10 +96,6 @@ struct IgemmParams {
   // shared memory plan (bytes)
   int plane_stride, a_stage_bytes, b_stage_bytes, nsa, nsb, tmem_cols;
   int box_planes;                // > 1: ONE TMA box carries all n_in_planes planes of an A tile (planes bh * bw * pitch apart)
-  int mma_planes;                // kMma == 2 instantiations: the two issuing warps split the PLANES of a tile (separate
-                                 // accumulators, both K = 16 halves each) instead of the K halves of every instruction
-  int b_boxes, b_box_rows;       // b_boxes > 0 (folded 3x3x3 tiles, depth-tap blocks adjacent in the pack): the weight tile
-                                 // of a tap arrives as b_boxes boxes of b_box_rows rows instead of one box per depth tap
   int nacc;                      // TMEM accumulator sets (>= 2: the epilogue of a tile overlaps the next tiles' MMAs; <= kMaxAccSets)
   int total_tiles;
 };
@@ -144,10 +141,9 @@ constexpr int kIgemmThreads = 192;  // marching / wgrad kernels: warps 0-3 epilo
 // per-channel accumulators. WITHOUT statistics -- every dgrad, the transposed convs, the PatchGAN stem -- a separate
 // instantiation drops that code and its registers (168 -> 120): ncu showed the output-heavy launches of that group
 // (transposed conv 64 -> 64: 2.1 GB written for 16 UMMAs per tile) bound by the epilogue's instruction stream, not by
-// HBM or L2 (profiles/r02g_deconv_pair.txt). It would also fit 16 epilogue warps (kFwdEpiWarpsWide); measured, that
-// does not pay (profiles/r02g_epi16.txt).
+// HBM or L2 (profiles/r02g_deconv_pair.txt). Sixteen epilogue warps for that instantiation were measured, removed: they
+// do not pay (profiles/r02g_epi16.txt).
 constexpr int kFwdEpiWarps = 8;
-constexpr int kFwdEpiWarpsWide = 16;
 constexpr int kFwdThreads = (kFwdEpiWarps + 3) * 32;  // warps 0-7 epilogue, 8 TMA producer (A), 9 MMA issuer, 10 TMA producer (B)
 constexpr int kFwdRedFloats = 2 * kFwdEpiWarps * 2 * 128 + 128;  // [parity][warp][sum|sumsq][128] + bias[128]
 
@@ -167,10 +163,9 @@ __device__ __forceinline__ IgemmTileCoord igemm_tile(const IgemmParams& P, int t
 
 // First tap of a full folded tile: every output plane's first contribution (kd = 0) overwrites its accumulator, so
 // the depth taps cannot share an instruction; same compile-time schedule, N = nt per UMMA.
-template <int ND, int PL, int kMma>
+template <int ND, int PL>
 __device__ __forceinline__ void issue_first_tap(uint32_t acc0, uint32_t a_tap, uint32_t a_hi, uint32_t b_lo0, uint32_t b_hi,
-                                                uint32_t ntc, uint32_t plane16, uint32_t kd_rows16, uint32_t idesc,
-                                                uint32_t koff, int half) {
+                                                uint32_t ntc, uint32_t plane16, uint32_t kd_rows16, uint32_t idesc) {
   constexpr int ndm1 = ND - 1;
 #pragma unroll
   for (int p_in = 0; p_in < PL + ndm1; ++p_in) {
@@ -182,12 +177,8 @@ __device__ __forceinline__ void issue_first_tap(uint32_t acc0, uint32_t a_tap, u
       const uint32_t d = acc0 + (uint32_t)o * ntc;
       const uint32_t a = a_tap + (uint32_t)p_in * plane16;
       const uint32_t b = b_lo0 + (uint32_t)(ndm1 - kd) * kd_rows16;
-      if (kMma == 2) {
-        umma_bf16_lohi(d, a + koff, a_hi, b + koff, b_hi, idesc, half ? 1u : (uint32_t)(kd != 0));
-      } else {
-        umma_bf16_lohi(d, a, a_hi, b, b_hi, idesc, (uint32_t)(kd != 0));
-        umma_bf16_lohi(d, a + 2, a_hi, b + 2, b_hi, idesc, 1u);
-      }
+      umma_bf16_lohi(d, a, a_hi, b, b_hi, idesc, (uint32_t)(kd != 0));
+      umma_bf16_lohi(d, a + 2, a_hi, b + 2, b_hi, idesc, 1u);
     }
   }
 }
@@ -199,10 +190,10 @@ template <int V> struct IntC { static constexpr int value = V; };
 // constant multiple of three warp-uniform strides on top of three bases and the compiler keeps the whole run in the
 // uniform datapath. The generic per-tile table (fs_* below) costs ~9 instructions per UMMA, most of them vector ->
 // uniform register moves: 113 cycles per N = 64 UMMA against ~50 for its operands (profiles/r02f_stem_fwd_ncu_summary.txt).
-template <int ND, int FOLD, int PL, int kMma>
+template <int ND, int FOLD, int PL>
 __device__ __forceinline__ void issue_folded_tap(uint32_t acc0, uint32_t a_tap, uint32_t a_hi, uint32_t b_lo0, uint32_t b_hi,
                                                  uint32_t ntc, uint32_t plane16, uint32_t kd_rows16,
-                                                 const uint32_t (&idesc_blk)[3], uint32_t koff) {
+                                                 const uint32_t (&idesc_blk)[3]) {
   constexpr int ndm1 = ND - 1;
 #pragma unroll
   for (int p_in = 0; p_in < PL + ndm1; ++p_in) {
@@ -215,32 +206,27 @@ __device__ __forceinline__ void issue_folded_tap(uint32_t acc0, uint32_t a_tap, 
       const uint32_t a = a_tap + (uint32_t)p_in * plane16;
       const uint32_t b = b_lo0 + (uint32_t)(ndm1 - (p_in - oa)) * kd_rows16;
       const uint32_t id = idesc_blk[ob - oa];
-      if (kMma == 2) {
-        umma_bf16_lohi(d, a + koff, a_hi, b + koff, b_hi, id, 1u);
-      } else {
-        umma_bf16_lohi(d, a, a_hi, b, b_hi, id, 1u);
-        umma_bf16_lohi(d, a + 2, a_hi, b + 2, b_hi, id, 1u);
-      }
+      umma_bf16_lohi(d, a, a_hi, b, b_hi, id, 1u);
+      umma_bf16_lohi(d, a + 2, a_hi, b + 2, b_hi, id, 1u);
     }
   }
 }
 
-// kMma = 2: TWO MMA-issuing warps. Every 32-channel K chunk of a tap is a pair of K = 16 UMMAs; warp kEpi + 1 issues
-// the first of each pair, warp kEpi + 2 the second, into the same accumulators. Why: the issue loop costs ~8
-// instructions per UMMA (each operand crosses from vector to uniform registers, R2UR), 113 cycles per N = 64 UMMA
+// kMma = 2: TWO MMA-issuing warps that split the PLANES of a tile, each on its own accumulators. The host launches it
+// for folded tiles only (launch_igemm: the four-plane schedule with three depth taps per UMMA). Why: the issue loop costs
+// ~8 instructions per UMMA (each operand crosses from vector to uniform registers, R2UR), 113 cycles per N = 64 UMMA
 // measured against ~50 for its shared-memory operands (profiles/r02f_stem_fwd_ncu_summary.txt), so every launch with
-// N <= 128 per instruction is bound by ONE thread's issue rate. Accumulation order between the two streams is
-// free, except that the second stream must not touch an accumulator before the first stream's overwriting UMMA
-// (first tap of a tile) has been issued: `first_bar`, one arrival per tile, orders exactly that (tcgen05 fences on
-// both sides; the tensor pipe executes in issue order). The stage / accumulator barriers count two commits.
-// Warp roles: 0 .. kEpi-1 epilogue, kEpi: TMA producer of the activation (A) stages, kEpi+1 (.. +kMma): MMA issuer(s),
-// last warp: TMA producer of the weight (B) ring. Two producers because ONE thread issuing every TMA operation bound the
+// N <= 128 per instruction is bound by ONE thread's issue rate. The stage / accumulator barriers count two commits.
+// (Two warps issuing the two K = 16 halves of every instruction into the SAME accumulators were 8-35 % slower,
+// profiles/r02g_mma2.txt: measured, removed.)
+// Warp roles: 0 .. kFwdEpiWarps-1 epilogue, kFwdEpiWarps: TMA producer of the activation (A) stages, kFwdEpiWarps+1
+// (.. +kMma): MMA issuer(s), last warp: TMA producer of the weight (B) ring. Two producers because ONE thread issuing every TMA operation bound the
 // launches with little MMA work per box: the stem forward needs 40 A + 64 B boxes per tile, ~290 cycles each
 // = the 30 k cycles per tile the launch took, against 16 k cycles of UMMAs (profiles/r02i_producer_ab.txt).
-template <int kEpi, bool kStats, int kMma = 1>
-__global__ void __launch_bounds__((kEpi + 2 + kMma) * 32, 1)
+template <bool kStats, int kMma>
+__global__ void __launch_bounds__((kFwdEpiWarps + 2 + kMma) * 32, 1)
 igemm_fwd_kernel(const __grid_constant__ IgemmParams P) {
-  static_assert(!kStats || kEpi == kFwdEpiWarps, "the statistics staging area is sized for kFwdEpiWarps warps");
+  constexpr int kEpi = kFwdEpiWarps;
   static_assert(kMma == 1 || kMma == 2, "one or two MMA-issuing warps");
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -252,10 +238,9 @@ igemm_fwd_kernel(const __grid_constant__ IgemmParams P) {
   const uint32_t bar_base = b_base + P.nsb * P.b_stage_bytes;  // 8-byte mbarriers
   // barrier layout: a_full[nsa] a_empty[nsa] b_full[nsb] b_empty[nsb] acc_full[kMaxAccSets] acc_empty[kMaxAccSets]
   const uint32_t a_full = bar_base, a_empty = a_full + 8 * P.nsa, b_full = a_empty + 8 * P.nsa,
-                 b_empty = b_full + 8 * P.nsb, acc_full = b_empty + 8 * P.nsb, acc_empty = acc_full + 8 * kMaxAccSets,
-                 first_bar = acc_empty + 8 * kMaxAccSets;   // [kMaxAccSets]: first tap of the tile issued (kMma == 2)
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(sm + (first_bar + 8 * kMaxAccSets - base));
-  float* red = reinterpret_cast<float*>(sm + (((first_bar + 8 * kMaxAccSets + 16 + 15) & ~15u) - base));  // kFwdRedFloats, 16-B aligned
+                 b_empty = b_full + 8 * P.nsb, acc_full = b_empty + 8 * P.nsb, acc_empty = acc_full + 8 * kMaxAccSets;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(sm + (acc_empty + 8 * kMaxAccSets - base));
+  float* red = reinterpret_cast<float*>(sm + (((acc_empty + 8 * kMaxAccSets + 16 + 15) & ~15u) - base));  // kFwdRedFloats, 16-B aligned
 
   const IgemmNTile NT = P.ntile[blockIdx.y];
   const int ntc = (NT.nt + 31) & ~31;  // TMEM columns per plane accumulator
@@ -264,9 +249,7 @@ igemm_fwd_kernel(const __grid_constant__ IgemmParams P) {
   if (threadIdx.x == 0) {
     for (int i = 0; i < P.nsa; ++i) { mbar_init(a_full + 8 * i, 1); mbar_init(a_empty + 8 * i, kMma); }
     for (int i = 0; i < P.nsb; ++i) { mbar_init(b_full + 8 * i, 1); mbar_init(b_empty + 8 * i, kMma); }
-    for (int i = 0; i < kMaxAccSets; ++i) {
-      mbar_init(acc_full + 8 * i, kMma); mbar_init(acc_empty + 8 * i, kEpi); mbar_init(first_bar + 8 * i, 1);
-    }
+    for (int i = 0; i < kMaxAccSets; ++i) { mbar_init(acc_full + 8 * i, kMma); mbar_init(acc_empty + 8 * i, kEpi); }
     fence_mbar_init();
   }
   if (warp == kEpi && lane == 0) {
@@ -279,7 +262,7 @@ igemm_fwd_kernel(const __grid_constant__ IgemmParams P) {
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = *tmem_slot;
-  const int pitch = P.kc * 2;
+  constexpr int pitch = kIgemmKc * 2;
 
   if (warp == kEpi) {
     // =========================== TMA producer: activation stages ===========================
@@ -295,7 +278,7 @@ igemm_fwd_kernel(const __grid_constant__ IgemmParams P) {
           const bool s1 = ch >= P.n_chunks_src0;
           const CUtensorMap* tm = &P.tm_src[s1 ? 1 : 0];
           const int grp = P.chunks_per_group ? ch / P.chunks_per_group : 0;
-          const int c0 = P.chunks_per_group ? (ch % P.chunks_per_group) * P.kc : (s1 ? ch - P.n_chunks_src0 : ch) * P.kc;
+          const int c0 = P.chunks_per_group ? (ch % P.chunks_per_group) * kIgemmKc : (s1 ? ch - P.n_chunks_src0 : ch) * kIgemmKc;
           const int nb5 = P.chunks_per_group ? T.nb * (P.n_chunks_total / P.chunks_per_group) + grp : T.nb;
           uint32_t dst = a_base + sa * P.a_stage_bytes;
           for (int at = 0; at < P.n_atiles; ++at) {
@@ -327,21 +310,17 @@ igemm_fwd_kernel(const __grid_constant__ IgemmParams P) {
       for (int t = blockIdx.x; t < P.total_tiles; t += gridDim.x) {
         for (int ch = 0; ch < P.n_chunks_total; ++ch) {
           const int grp = P.chunks_per_group ? ch / P.chunks_per_group : 0;
-          const int wk = (P.chunks_per_group ? ch % P.chunks_per_group : ch) * P.kc;
+          const int wk = (P.chunks_per_group ? ch % P.chunks_per_group : ch) * kIgemmKc;
           const IgemmTap* taps = P.taps + (P.chunks_per_group ? grp : NT.tapset) * P.ntaps;
           for (int tp = 0; tp < P.ntaps; ++tp) {
             mbar_wait(b_empty + 8 * sb, pb ^ 1);
             mbar_expect_tx(b_full + 8 * sb, b_bytes);
             const int brow = (taps[tp].wblock + NT.wblock_add) * P.b_block_rows + NT.n0;
-            if (P.b_boxes) {
-              for (int j = 0; j < P.b_boxes; ++j)
-                tma_load_2d(b_base + sb * P.b_stage_bytes + j * P.b_box_rows * pitch, &P.tm_w, b_full + 8 * sb, wk,
-                            brow + j * P.b_box_rows);
-              if (++sb == P.nsb) { sb = 0; pb ^= 1; }
-              continue;
-            }
             tma_load_2d(b_base + sb * P.b_stage_bytes, &P.tm_w, b_full + 8 * sb, wk, brow);
-            if (P.kd_fold) {   // the other depth-tap blocks of the folded tile (TMA boxes hold <= 256 rows)
+            // the other depth-tap blocks of the folded tile, one box each (TMA boxes hold <= 256 rows). The blocks of a
+            // 3x3x3 tile are adjacent in the pack; one merged box for them measured neutral, removed
+            // (profiles/r02i_wbox_ab.txt: these launches are not bound by the producer's issue rate).
+            if (P.kd_fold) {
               for (int j = 1; j < P.fold_nd; ++j)
                 tma_load_2d(b_base + sb * P.b_stage_bytes + j * NT.nt * pitch, &P.tm_w, b_full + 8 * sb, wk,
                             brow + j * P.fold_row_step);
@@ -355,14 +334,10 @@ igemm_fwd_kernel(const __grid_constant__ IgemmParams P) {
   } else if (warp >= kEpi + 1) {
     // =========================== MMA issuer(s): warps kEpi+1 .. kEpi+kMma ===========================
     // The whole warp walks the pipeline (uniform control flow); one elected lane issues.
-    const bool split_planes = kMma == 2 && P.mma_planes != 0;
-    const int ph = kMma == 2 ? warp - (kEpi + 1) : 0;        // this warp's index among the issuers
-    const int half = split_planes ? 0 : ph;                  // which UMMA of every K = 16 pair this warp issues (K-half mode)
-    const uint32_t koff = 2u * (uint32_t)half;               // its K offset in 16-byte units
-    const uint32_t swz = P.kc == 32 ? SWZ_64B : (P.kc == 16 ? SWZ_32B : SWZ_128B);
+    const int ph = kMma == 2 ? warp - (kEpi + 1) : 0;        // this warp's index among the issuers (its half of the planes)
     const uint32_t idesc = make_idesc_bf16(128, NT.nt, 0, 0);
-    const uint32_t a_hi = (uint32_t)(make_smem_desc(0, 16, P.bw * pitch, swz) >> 32);
-    const uint32_t b_hi = (uint32_t)(make_smem_desc(0, 16, 8 * pitch, swz) >> 32);
+    const uint32_t a_hi = (uint32_t)(make_smem_desc(0, 16, P.bw * pitch, SWZ_64B) >> 32);
+    const uint32_t b_hi = (uint32_t)(make_smem_desc(0, 16, 8 * pitch, SWZ_64B) >> 32);
     const uint32_t lbo_lo = 1u << 16;  // LBO field (16 bytes) lives in the low word
     const uint32_t plane16 = (uint32_t)P.plane_stride >> 4;
     const bool leader = elect_one();
@@ -385,7 +360,7 @@ igemm_fwd_kernel(const __grid_constant__ IgemmParams P) {
                         : (P.fold_nd == 3 && fold == 3 && T.planes == 4) ? 1
                         : (P.fold_nd == 3 && fold == 2 && T.planes == 2) ? 2
                         : (P.fold_nd == 2 && fold == 2 && T.planes == 4) ? 3 : 0;
-      if (fold && sched == 0) {
+      if (fold && sched == 0 && ph == 0) {   // (a second issuer leaves such tiles to the first)
 #pragma unroll
         for (int p_in = 0; p_in < 6; ++p_in) {
 #pragma unroll
@@ -416,54 +391,44 @@ igemm_fwd_kernel(const __grid_constant__ IgemmParams P) {
         for (int tp = 0; tp < P.ntaps; ++tp) {
           mbar_wait(b_full + 8 * sb, pb);
           tc_fence_after();
-          const bool first_tap = (ch | tp) == 0;
-          if (kMma == 2 && !split_planes && first_tap && half == 1) {
-            // the first stream's overwriting UMMAs of this tile must be in the pipe before anything accumulates
-            mbar_wait(first_bar + 8 * slot, pacc);
-            tc_fence_after();
-          }
           if (leader && P.kd_fold) {
             const IgemmTap Tp = P.taps[tbase + tp];
             const uint32_t a_tap = lbo_lo | ((a_stage + Tp.row_off * pitch) >> 4);
             const uint32_t b_lo0 = lbo_lo | ((b_base + sb * P.b_stage_bytes) >> 4);
-            if (split_planes && sched != 0) {
+            if (kMma == 2 && sched != 0) {
               // plane-split issuers: each warp runs the schedule of HALF the tile's planes on its own accumulators --
               // (3, 3, 4) -> two (3, 2, 2) halves, (3, 2, 2) -> two (3, 1, 1), (2, 2, 4) -> two (2, 2, 2)
               const uint32_t nh = sched == 2 ? 1u : 2u;                       // output planes per issuer
               const uint32_t accp = acc0 + (uint32_t)ph * nh * (uint32_t)ntc, a_p = a_tap + (uint32_t)ph * nh * plane16;
               if ((ch | tp) != 0) {
-                if (sched == 1) issue_folded_tap<3, 2, 2, 1>(accp, a_p, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc_blk, 0u);
-                else if (sched == 2) issue_folded_tap<3, 1, 1, 1>(accp, a_p, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc_blk, 0u);
-                else issue_folded_tap<2, 2, 2, 1>(accp, a_p, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc_blk, 0u);
+                if (sched == 1) issue_folded_tap<3, 2, 2>(accp, a_p, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc_blk);
+                else if (sched == 2) issue_folded_tap<3, 1, 1>(accp, a_p, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc_blk);
+                else issue_folded_tap<2, 2, 2>(accp, a_p, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc_blk);
               } else {
-                if (sched == 1) issue_first_tap<3, 2, 1>(accp, a_p, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc, 0u, 0);
-                else if (sched == 2) issue_first_tap<3, 1, 1>(accp, a_p, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc, 0u, 0);
-                else issue_first_tap<2, 2, 1>(accp, a_p, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc, 0u, 0);
+                if (sched == 1) issue_first_tap<3, 2>(accp, a_p, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc);
+                else if (sched == 2) issue_first_tap<3, 1>(accp, a_p, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc);
+                else issue_first_tap<2, 2>(accp, a_p, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc);
               }
-            } else if (split_planes && ph == 1) {
+            } else if (kMma == 2 && ph == 1) {
               // ragged tile: the first issuer runs the whole table, this one only commits
             } else if ((ch | tp) != 0 && sched != 0) {
               // full tile of one of the three shapes the step uses: compile-time schedule
-              if (sched == 1) issue_folded_tap<3, 3, 4, kMma>(acc0, a_tap, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc_blk, koff);
-              else if (sched == 2) issue_folded_tap<3, 2, 2, kMma>(acc0, a_tap, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc_blk, koff);
-              else issue_folded_tap<2, 2, 4, kMma>(acc0, a_tap, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc_blk, koff);
+              if (sched == 1) issue_folded_tap<3, 3, 4>(acc0, a_tap, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc_blk);
+              else if (sched == 2) issue_folded_tap<3, 2, 2>(acc0, a_tap, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc_blk);
+              else issue_folded_tap<2, 2, 4>(acc0, a_tap, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc_blk);
             } else if ((ch | tp) != 0) {
               // any other tile (ragged depth, other fold shapes): the per-tile schedule table (fs_*)
 #pragma unroll
               for (int e = 0; e < 12; ++e) {
                 if ((fs_valid >> e) & 1u) {
-                  if (kMma == 2 && !split_planes) {
-                    umma_bf16_lohi(acc0 + fs_d[e], a_tap + fs_a[e] + koff, a_hi, b_lo0 + fs_b[e] + koff, b_hi, fs_i[e], 1u);
-                  } else {
-                    umma_bf16_lohi(acc0 + fs_d[e], a_tap + fs_a[e], a_hi, b_lo0 + fs_b[e], b_hi, fs_i[e], 1u);
-                    umma_bf16_lohi(acc0 + fs_d[e], a_tap + fs_a[e] + 2, a_hi, b_lo0 + fs_b[e] + 2, b_hi, fs_i[e], 1u);
-                  }
+                  umma_bf16_lohi(acc0 + fs_d[e], a_tap + fs_a[e], a_hi, b_lo0 + fs_b[e], b_hi, fs_i[e], 1u);
+                  umma_bf16_lohi(acc0 + fs_d[e], a_tap + fs_a[e] + 2, a_hi, b_lo0 + fs_b[e] + 2, b_hi, fs_i[e], 1u);
                 }
               }
             } else if (sched != 0) {
-              if (sched == 1) issue_first_tap<3, 4, kMma>(acc0, a_tap, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc, koff, half);
-              else if (sched == 2) issue_first_tap<3, 2, kMma>(acc0, a_tap, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc, koff, half);
-              else issue_first_tap<2, 4, kMma>(acc0, a_tap, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc, koff, half);
+              if (sched == 1) issue_first_tap<3, 4>(acc0, a_tap, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc);
+              else if (sched == 2) issue_first_tap<3, 2>(acc0, a_tap, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc);
+              else issue_first_tap<2, 4>(acc0, a_tap, a_hi, b_lo0, b_hi, (uint32_t)ntc, plane16, kd_rows16, idesc);
             } else {
               // first tap of the tile: each output plane's first contribution (kd = 0) overwrites
               for (int p_in = 0; p_in < n_pin; ++p_in) {
@@ -473,12 +438,8 @@ igemm_fwd_kernel(const __grid_constant__ IgemmParams P) {
                 for (int o = o_lo; o <= o_hi; ++o) {
                   const int kd = p_in - o;
                   const uint32_t b_lo = b_lo0 + (uint32_t)(ndm1 - kd) * kd_rows16;
-                  if (kMma == 2 && !split_planes) {
-                    umma_bf16_lohi(acc0 + o * ntc, a_lo + koff, a_hi, b_lo + koff, b_hi, idesc, half ? 1u : (uint32_t)(kd != 0));
-                  } else {
-                    umma_bf16_lohi(acc0 + o * ntc, a_lo, a_hi, b_lo, b_hi, idesc, (uint32_t)(kd != 0));
-                    umma_bf16_lohi(acc0 + o * ntc, a_lo + 2, a_hi, b_lo + 2, b_hi, idesc, 1u);
-                  }
+                  umma_bf16_lohi(acc0 + o * ntc, a_lo, a_hi, b_lo, b_hi, idesc, (uint32_t)(kd != 0));
+                  umma_bf16_lohi(acc0 + o * ntc, a_lo + 2, a_hi, b_lo + 2, b_hi, idesc, 1u);
                 }
               }
             }
@@ -491,36 +452,19 @@ igemm_fwd_kernel(const __grid_constant__ IgemmParams P) {
             const uint32_t acc = (ch | tp) != 0;
             // one branch per tap, not per plane: the planes of a tap are then one straight run of UMMAs (every branch
             // in between makes the compiler move all seven operands to uniform registers again)
-            auto planes = [&](auto pl, auto ks) {
+            auto planes = [&](auto pl) {
               constexpr int PL = decltype(pl)::value;
 #pragma unroll
               for (int o = 0; o < PL; ++o) {
-                // plane-split issuers: even plane counts are halved between the two warps, odd ones stay with the first
-                if (split_planes && ((PL % 2 == 0) ? (o / (PL / 2) != ph) : (ph != 0))) continue;
-                if (kMma == 2 && !split_planes) {
-                  umma_bf16_lohi(acc0 + o * ntc, a_lo + o * plane16 + koff, a_hi, b_lo + koff, b_hi, idesc, half ? 1u : acc);
-                } else {
-                  // K = 16 steps of the chunk: two for 32-channel chunks, four for 64-channel chunks (128-byte rows)
-#pragma unroll
-                  for (int k = 0; k < decltype(ks)::value; ++k)
-                    umma_bf16_lohi(acc0 + o * ntc, a_lo + o * plane16 + 2 * k, a_hi, b_lo + 2 * k, b_hi, idesc, k == 0 ? acc : 1u);
-                }
+                umma_bf16_lohi(acc0 + o * ntc, a_lo + o * plane16, a_hi, b_lo, b_hi, idesc, acc);
+                umma_bf16_lohi(acc0 + o * ntc, a_lo + o * plane16 + 2, a_hi, b_lo + 2, b_hi, idesc, 1u);
               }
             };
-            if (P.kc == 64) {
-              if (T.planes == 4) planes(IntC<4>{}, IntC<4>{});
-              else if (T.planes == 2) planes(IntC<2>{}, IntC<4>{});
-              else if (T.planes == 1) planes(IntC<1>{}, IntC<4>{});
-              else planes(IntC<3>{}, IntC<4>{});
-            } else if (T.planes == 4) planes(IntC<4>{}, IntC<2>{});
-            else if (T.planes == 2) planes(IntC<2>{}, IntC<2>{});
-            else if (T.planes == 1) planes(IntC<1>{}, IntC<2>{});
-            else planes(IntC<3>{}, IntC<2>{});
+            if (T.planes == 4) planes(IntC<4>{});
+            else if (T.planes == 2) planes(IntC<2>{});
+            else if (T.planes == 1) planes(IntC<1>{});
+            else planes(IntC<3>{});
             umma_commit(b_empty + 8 * sb);
-          }
-          if (kMma == 2 && !split_planes && first_tap && half == 0) {
-            tc_fence_before();
-            if (leader) mbar_arrive(first_bar + 8 * slot);
           }
           __syncwarp();
           if (++sb == P.nsb) { sb = 0; pb ^= 1; }

@@ -53,7 +53,6 @@ struct MarchParams {
                                     // against weight columns packed as fp16, UB_PACK_F16_SRC0)
   NormActArgs tf;
   int tf_f16;                       // the transformed chunk is an fp16 operand (its weight columns are packed as fp16)
-  int mma2;                         // single-CTA, untransformed variants: TWO MMA-issuing warps, planes alternating
 };
 
 constexpr int kMarchPlaneBytes = 12288;   // 180 rows x 64 B, padded to a multiple of 1024
@@ -71,12 +70,10 @@ constexpr int kMarchThreadsTf = kMarchThreads + kMarchTfThreads;
 
 // One MMA issuer of the single-CTA, untransformed kernel taking planes p_first + me, + step, ...: ring slot, stage and
 // barrier phases follow from the plane index alone, so several issuers need no shared state.
-template <bool kPair>
 __device__ __forceinline__ void march_issue_planes(const MarchParams& P, int me, int step, int p_first, int p_last, int nch,
                                                    uint32_t tmem, uint32_t w_base, uint32_t a_base, uint32_t w_full,
                                                    uint32_t a_full, uint32_t a_empty, uint32_t acc_full, uint32_t acc_empty) {
-  constexpr int kWTile = kPair ? kMarchWTileBytes / 2 : kMarchWTileBytes;   // this CTA's share of a weight tile
-  const uint32_t idesc_bf = make_idesc_bf16(kPair ? 256 : 128, 96, 0, 0);
+  const uint32_t idesc_bf = make_idesc_bf16(128, 96, 0, 0);
   const uint32_t idesc_h = idesc_f16_operands(idesc_bf);
   const uint32_t a_hi = (uint32_t)(make_smem_desc(0, 16, 10 * 64, SWZ_64B) >> 32);
   const uint32_t b_hi = (uint32_t)(make_smem_desc(0, 16, 8 * 64, SWZ_64B) >> 32);
@@ -99,30 +96,21 @@ __device__ __forceinline__ void march_issue_planes(const MarchParams& P, int me,
       if (leader) {
         const uint32_t idesc = c < n_f16 ? idesc_h : idesc_bf;
         const uint32_t a_lo = lbo_lo | ((a_base + sa * kMarchPlaneBytes) >> 4);
-        const uint32_t b_lo = lbo_lo | ((w_base + c * 9 * kWTile) >> 4);
+        const uint32_t b_lo = lbo_lo | ((w_base + c * 9 * kMarchWTileBytes) >> 4);
 #pragma unroll
         for (int kh = 0; kh < 3; ++kh)
 #pragma unroll
           for (int kw = 0; kw < 3; ++kw) {
             const uint32_t ao = (uint32_t)((kh * 10 + kw) * 64) >> 4;
-            const uint32_t bo = (uint32_t)((kh * 3 + kw) * kWTile) >> 4;
-            if (kPair) {
-              umma_bf16_lohi_pair(acc, a_lo + ao, a_hi, b_lo + bo, b_hi, idesc, (uint32_t)((c | kh | kw) != 0));
-              umma_bf16_lohi_pair(acc, a_lo + ao + 2, a_hi, b_lo + bo + 2, b_hi, idesc, 1u);
-            } else {
-              umma_bf16_lohi(acc, a_lo + ao, a_hi, b_lo + bo, b_hi, idesc, (uint32_t)((c | kh | kw) != 0));
-              umma_bf16_lohi(acc, a_lo + ao + 2, a_hi, b_lo + bo + 2, b_hi, idesc, 1u);
-            }
+            const uint32_t bo = (uint32_t)((kh * 3 + kw) * kMarchWTileBytes) >> 4;
+            umma_bf16_lohi(acc, a_lo + ao, a_hi, b_lo + bo, b_hi, idesc, (uint32_t)((c | kh | kw) != 0));
+            umma_bf16_lohi(acc, a_lo + ao + 2, a_hi, b_lo + bo + 2, b_hi, idesc, 1u);
           }
-        if (kPair) umma_commit_pair(a_empty + 8 * sa);
-        else umma_commit(a_empty + 8 * sa);
+        umma_commit(a_empty + 8 * sa);
       }
       __syncwarp();
     }
-    if (leader) {
-      if (kPair) umma_commit_pair(acc_full + 8 * slot);
-      else umma_commit(acc_full + 8 * slot);
-    }
+    if (leader) umma_commit(acc_full + 8 * slot);
     __syncwarp();
   }
 }
@@ -137,10 +125,12 @@ __device__ __forceinline__ void march_issue_planes(const MarchParams& P, int me,
 // a_loc[stage] (pair mode: each CTA waits for its own plane), the transform warps hand the stage to the MMA thread
 // through a_ready[stage] in the leader CTA (one arrival per CTA). Untransformed chunks keep the a_full path. A
 // stage alternates between the two paths, so the barrier phases are tracked per stage in bit masks.
-// mma2 (!kTf, !kPair, opt-in): warp kMmaWarp + 1 is a second MMA issuer. The two warps take alternating planes -- different
+// !kPair && !kTf: warp kMmaWarp + 1 is a second MMA issuer. The two warps take alternating planes -- different
 // accumulator slots and different A stages, so nothing orders them against each other -- and one warp's per-plane
-// hand-off (two barrier waits, two fences, two commits) runs while the other one's UMMAs are in the pipe. Unlike the
-// generic kernel's UB_MMA2 (two warps feeding the SAME accumulators) the streams are independent.
+// hand-off (two barrier waits, two fences, two commits) runs while the other one's UMMAs are in the pipe. Measured
+// (profiles/r02j_march_mma2.txt): one-chunk 32 -> 32 forward 0.875 -> 0.71 ms, its dgrad 0.85 -> 0.70, 24 -> 32
+// 0.85 -> 0.68, three chunks without CTA pairs 2.18 -> 2.05. In the CTA-pair kernel a second issuer measured neutral
+// (profiles/r02j_march_pair_mma2.txt), removed: warp kMmaWarp + 1 idles there.
 constexpr int kMarchThreads2 = kMarchThreads + 32;
 template <bool kNormBwd, bool kPair, bool kTf>
 __global__ void __launch_bounds__(kTf ? kMarchThreadsTf : kMarchThreads2, 1)
@@ -249,9 +239,8 @@ igemm_march_kernel(const __grid_constant__ MarchParams P) {
     __syncwarp();
   } else if (warp == kMmaWarp) {
     // =========================== MMA issuer (leader CTA only in pair mode) ===========================
-    if (!kTf && P.mma2) {
-      if (rank == 0)
-        march_issue_planes<kPair>(P, 0, 2, p_first, p_last, nch, tmem, w_base, a_base, w_full, a_full, a_empty, acc_full, acc_empty);
+    if (!kPair && !kTf) {
+      march_issue_planes(P, 0, 2, p_first, p_last, nch, tmem, w_base, a_base, w_full, a_full, a_empty, acc_full, acc_empty);
     } else if (rank == 0) {
       const uint32_t idesc_bf = make_idesc_bf16(kPair ? 256 : 128, 96, 0, 0);
       const uint32_t idesc_h = idesc_f16_operands(idesc_bf);
@@ -316,9 +305,8 @@ igemm_march_kernel(const __grid_constant__ MarchParams P) {
       }
     }
   } else if (!kTf && warp == kMmaWarp + 1) {
-    // =========================== second MMA issuer (mma2): odd planes ===========================
-    if (P.mma2 && rank == 0) march_issue_planes<kPair>(P, 1, 2, p_first, p_last, nch, tmem, w_base, a_base, w_full, a_full, a_empty,
-                                                       acc_full, acc_empty);
+    // =========================== second MMA issuer (single CTA): odd planes ===========================
+    if (!kPair) march_issue_planes(P, 1, 2, p_first, p_last, nch, tmem, w_base, a_base, w_full, a_full, a_empty, acc_full, acc_empty);
   } else if (kTf && warp >= kMarchEpiWarps) {
     // =========================== operand transform (warps 8-9) ===========================
     const int t = (int)threadIdx.x - kMarchEpiWarps * 32;

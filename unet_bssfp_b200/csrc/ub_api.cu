@@ -42,7 +42,7 @@ static std::atomic<long long> g_launches{0};
     if (e_ != cudaSuccess) return fail(-3, "kernel launch failed: %s", cudaGetErrorString(e_)); \
   } while (0)
 
-// A/B switches for measurements (read on every call: tests and tools flip them inside one process)
+// Switches to a reference path (read on every call: tests and tools flip them inside one process)
 static bool env_flag(const char* name) {
   const char* v = getenv(name);
   return v && atoi(v) != 0;
@@ -292,44 +292,25 @@ static int opt_in_smem(SmemOptIn& st, const void* fn, const char* what) {
   return 0;
 }
 
-// Channels per K chunk of the generic kernel. The TMA unit fetches ~one row per 5 cycles per SM whatever its length
-// (tools/tma_rate.cu); 64-channel chunks -- 128-byte rows, four K = 16 UMMAs per chunk -- halve the rows of a layer
-// with >= 64 input channels. Built for the transposed convs (no halo, so the wider stages fit) and measured there
-// (profiles/r02j_kc64_ab.txt): 64 -> 64 forward 0.496 -> 0.507 ms (bound by its 2.1 GB of output stores, not by the
-// loads), 128 -> 64 0.083 -> 0.078, dgrads equal or slower (one-plane tiles). Opt-in: UB_KC64 bit 0 forward, bit 1 dgrad.
-static int chunk_channels(int kind, int channels, int dir) {
-  static const int mask = getenv("UB_KC64") ? atoi(getenv("UB_KC64")) : 0;
-  return ((mask >> dir) & 1) && kind == UB_DECONV_K2S2 && channels % 64 == 0 ? 64 : 32;
-}
+// K chunks of the generic kernel are kIgemmKc = 32 channels. 64-channel chunks (128-byte rows, half the TMA rows) were
+// measured on the transposed convs (profiles/r02j_kc64_ab.txt): 64 -> 64 forward 0.496 -> 0.507 ms (bound by its 2.1 GB
+// of output stores, not by the loads), 128 -> 64 0.083 -> 0.078, dgrads equal or slower (one-plane tiles); removed.
 
 // Planes per activation TMA box of the generic kernel: all the planes of a tile in ONE box (the producer thread's
-// issue rate bounds the launches with little MMA work per box); UB_PLANE_BOX=0: one box per plane, as before.
+// issue rate bounds the launches with little MMA work per box). One box per plane for every shape was measured
+// (profiles/r02i_producer_ab.txt) and removed; it remains for the shapes rejected here.
 static int plane_box(const IgemmParams& P) {
-  static const bool on = !(getenv("UB_PLANE_BOX") && atoi(getenv("UB_PLANE_BOX")) == 0);
-  if (!on || P.n_in_planes <= 1 || P.n_in_planes * P.in_stride > 256) return 1;
+  if (P.n_in_planes <= 1 || P.n_in_planes * P.in_stride > 256) return 1;
   // several A tiles per stage: every tile's box must start on a 128-byte boundary
-  if (P.n_atiles > 1 && (P.n_in_planes * P.bh * P.bw * P.kc * 2) % 128 != 0) return 1;
+  if (P.n_atiles > 1 && (P.n_in_planes * P.bh * P.bw * kIgemmKc * 2) % 128 != 0) return 1;
   return P.n_in_planes;
-}
-
-// Folded 3x3x3 tiles: the three depth-tap blocks of a (chunk, kh, kw) weight tile are adjacent rows of the pack
-// (fold_row_step == nt), so the tile can arrive as ONE TMA box of 3 * nt rows (two boxes beyond 256 rows) instead of
-// three. Measured neutral on every 3x3x3 shape of the step (profiles/r02i_wbox_ab.txt: these launches are not bound
-// by the producer's issue rate), so it stays opt-in: UB_WBOX_MERGE=1.
-static void merged_weight_boxes(IgemmParams& P, int nt) {
-  static const bool on = getenv("UB_WBOX_MERGE") && atoi(getenv("UB_WBOX_MERGE")) != 0;
-  P.b_boxes = 0; P.b_box_rows = 0;
-  if (!on || !P.kd_fold || P.fold_nd != 3 || P.fold_row_step != nt) return;
-  const int rows = 3 * nt, nb = cdiv(rows, 256);
-  if (rows % nb != 0 || (rows / nb) % 8 != 0) return;
-  P.b_boxes = nb; P.b_box_rows = rows / nb;
 }
 
 // Fill the smem plan / grid once the geometry fields of P are set. nt_max = widest N tile.
 // The kernel is persistent with one CTA per SM: the whole shared memory goes to the TMA rings.
 static int finish_plan(IgemmPlan* pl, int nt_max) {
   IgemmParams& P = pl->P;
-  const int pitch = P.kc * 2;
+  const int pitch = kIgemmKc * 2;
   P.box_planes = plane_box(P);
   // a multi-plane box writes its planes back to back; the swizzle is a function of the absolute shared-memory address
   // (tools/probe_umma.cu), so a plane may start at any multiple of 128 bytes
@@ -352,13 +333,11 @@ static int finish_plan(IgemmPlan* pl, int nt_max) {
   if (pl->smem < 120 * 1024) pl->smem = 120 * 1024;   // never two CTAs on one SM (persistent: one per SM)
   const int set_cols = P.td * align_up(nt_max, 32);
   if (set_cols > 512) return fail(-2, "igemm TMEM plan too large: %d columns", set_cols);
-  // Two accumulator sets: the epilogue of a tile overlaps the next tile's MMAs. The kernel takes up to kMaxAccSets
-  // (UB_NACC_MAX=4); measured on the narrow-tile launches (1x1x1 head, stem forward / dgrad, d2: <= 128 columns per
-  // set) four sets change nothing (profiles/r02g_nacc.txt) -- those launches are bound by the epilogue's per-tile
-  // instruction count (statistics transpose) or the MMA thread's issue rate, not by the hand-off depth.
-  static const int nacc_max = getenv("UB_NACC_MAX") ? atoi(getenv("UB_NACC_MAX")) : 2;
+  // Two accumulator sets: the epilogue of a tile overlaps the next tile's MMAs. Four sets were measured on the
+  // narrow-tile launches (1x1x1 head, stem forward / dgrad, d2: <= 128 columns per set) and changed nothing
+  // (profiles/r02g_nacc.txt; removed) -- those launches are bound by the epilogue's per-tile instruction count
+  // (statistics transpose) or the MMA thread's issue rate, not by the hand-off depth.
   P.nacc = 512 / set_cols;
-  if (P.nacc > nacc_max) P.nacc = nacc_max;
   if (P.nacc > kMaxAccSets) P.nacc = kMaxAccSets;
   if (P.nacc < 1) P.nacc = 1;
   P.tmem_cols = next_pow2_cols(P.nacc * set_cols);
@@ -373,52 +352,26 @@ static int finish_plan(IgemmPlan* pl, int nt_max) {
   return 0;
 }
 
-static int launch_igemm_mma2(const IgemmPlan& pl, cudaStream_t st) {
-  static SmemOptIn opt[5];
-    // two MMA-issuing warps (see igemm_fwd.cuh)
-    if (pl.P.stats != nullptr) {
-      if (int e = opt_in_smem(opt[3], (const void*)igemm_fwd_kernel<kFwdEpiWarps, true, 2>, "igemm_fwd")) return e;
-      igemm_fwd_kernel<kFwdEpiWarps, true, 2><<<pl.grid, (kFwdEpiWarps + 4) * 32, pl.smem, st>>>(pl.P);
-    } else {
-      if (int e = opt_in_smem(opt[4], (const void*)igemm_fwd_kernel<kFwdEpiWarps, false, 2>, "igemm_fwd")) return e;
-      igemm_fwd_kernel<kFwdEpiWarps, false, 2><<<pl.grid, (kFwdEpiWarps + 4) * 32, pl.smem, st>>>(pl.P);
-    }
-    UB_LAUNCH_CHECK();
-    return 0;
-}
-
 static int launch_igemm(const IgemmPlan& pl, cudaStream_t st) {
-  // three instantiations: with statistics (8 epilogue warps, 64 accumulator registers per thread), and without
-  // statistics with 8 (default) or 16 (UB_EPI16=1) epilogue warps. Measured (profiles/r02g_epi16.txt): dropping the
-  // statistics code alone takes the transposed conv 64 -> 64 from 0.568 to 0.503 ms and the stem dgrad from 0.69 to
-  // 0.64 ms (120 instead of 168 registers); sixteen warps add little there (0.486) and cost elsewhere (32 -> 96-column
-  // dgrad 2.39 -> 2.47 ms, stem dgrad 0.70), so eight it stays.
-  static SmemOptIn opt[5];
-  static const bool epi16 = getenv("UB_EPI16") && atoi(getenv("UB_EPI16")) != 0;
-  static const bool mma2 = getenv("UB_MMA2") && atoi(getenv("UB_MMA2")) != 0;
-  // Two issuing warps that split the PLANES of a tile (independent accumulators, igemm_fwd.cuh `mma_planes`). Measured per
-  // shape (profiles/r02j_fwd_mma_planes.txt): the four-plane tiles with three depth taps per UMMA -- the 64-channel 3x3x3
+  // Instantiations by statistics: with them (forward convs in front of a norm: 64 accumulator registers per epilogue
+  // thread) and without. Measured (profiles/r02g_epi16.txt): dropping the statistics code alone takes the transposed
+  // conv 64 -> 64 from 0.568 to 0.503 ms and the stem dgrad from 0.69 to 0.64 ms (120 instead of 168 registers);
+  // sixteen epilogue warps add little there (0.486) and cost elsewhere (32 -> 96-column dgrad 2.39 -> 2.47 ms, stem
+  // dgrad 0.70): measured, removed.
+  // Two issuing warps that split the PLANES of a tile (kMma = 2, independent accumulators). Measured per shape
+  // (profiles/r02j_fwd_mma_planes.txt): the four-plane tiles with three depth taps per UMMA -- the 64-channel 3x3x3
   // layers -- gain 6-9 % (64 -> 64 @64^3 forward 0.365 -> 0.341 ms, dgrad 0.357 -> 0.325, 64+64 -> 64 0.679 -> 0.640,
   // 32 -> 64 0.210 -> 0.195); two-plane tiles (128 channels, the 96-column dgrad) do not move, the stem, the transposed
-  // convs, the 1x1x1 head and the 8^3 level lose 2-20 %. So: on for that schedule only. UB_MMA_PLANES=0: off, 2: everywhere.
-  static const int mma_planes_env = getenv("UB_MMA_PLANES") ? atoi(getenv("UB_MMA_PLANES")) : 1;
-  const bool mma_planes = mma_planes_env == 2 ? pl.P.td >= 2
-                                              : (mma_planes_env == 1 && pl.P.kd_fold == 3 && pl.P.fold_nd == 3 && pl.P.td == 4);
-  if ((mma2 || mma_planes) && pl.P.kc == 32) {
-    IgemmPlan plm = pl;
-    plm.P.mma_planes = (!mma2 && mma_planes) ? 1 : 0;
-    return launch_igemm_mma2(plm, st);
-  }
-  if (pl.P.stats != nullptr) {
-    if (int e = opt_in_smem(opt[0], (const void*)igemm_fwd_kernel<kFwdEpiWarps, true>, "igemm_fwd")) return e;
-    igemm_fwd_kernel<kFwdEpiWarps, true><<<pl.grid, (kFwdEpiWarps + 3) * 32, pl.smem, st>>>(pl.P);
-  } else if (epi16) {
-    if (int e = opt_in_smem(opt[1], (const void*)igemm_fwd_kernel<kFwdEpiWarpsWide, false>, "igemm_fwd")) return e;
-    igemm_fwd_kernel<kFwdEpiWarpsWide, false><<<pl.grid, (kFwdEpiWarpsWide + 3) * 32, pl.smem, st>>>(pl.P);
-  } else {
-    if (int e = opt_in_smem(opt[2], (const void*)igemm_fwd_kernel<kFwdEpiWarps, false>, "igemm_fwd")) return e;
-    igemm_fwd_kernel<kFwdEpiWarps, false><<<pl.grid, (kFwdEpiWarps + 3) * 32, pl.smem, st>>>(pl.P);
-  }
+  // convs, the 1x1x1 head and the 8^3 level lose 2-20 %. So: that schedule only (the other choices measured, removed).
+  const int stats = pl.P.stats != nullptr ? 1 : 0;
+  const int mma2 = pl.P.kd_fold == 3 && pl.P.fold_nd == 3 && pl.P.td == 4 ? 1 : 0;
+  typedef void (*IgemmFn)(const IgemmParams);
+  static const IgemmFn fns[2][2] = {{igemm_fwd_kernel<false, 1>, igemm_fwd_kernel<false, 2>},
+                                    {igemm_fwd_kernel<true, 1>, igemm_fwd_kernel<true, 2>}};
+  static SmemOptIn opt[2][2];
+  const IgemmFn fn = fns[stats][mma2];
+  if (int e = opt_in_smem(opt[stats][mma2], (const void*)fn, "igemm_fwd")) return e;
+  fn<<<pl.grid, (kFwdEpiWarps + 3 + mma2) * 32, pl.smem, st>>>(pl.P);
   UB_LAUNCH_CHECK();
   return 0;
 }
@@ -501,12 +454,10 @@ static int launch_march(const void* src0, int c0p, const void* src1, int c1p, in
   P.Nb = n; P.D = D; P.H = H; P.W = W;
   march_geometry(n, D, H, W, &P.tiles_w, &P.tiles_h, &P.nseg, &P.seg_len);
   P.out = out; P.bias = bias; P.bias_n = bias_n; P.stats = stats;
-  // CTA pairs (cta_group::2) whenever the w tiles pair up; UB_MARCH_PAIR=0 forces the single-CTA kernel
-  static const bool pair_enabled = !(getenv("UB_MARCH_PAIR") && atoi(getenv("UB_MARCH_PAIR")) == 0);
-  // (a plane must be long enough to amortise the cross-CTA barrier traffic: measured on B200 at 8x128^3,
-  // 1 K chunk 805 vs 1200 TFLOP/s single-CTA, 2 chunks 1374 vs 1330, 3 chunks 1576 vs 1360)
-  static const int pair_min_chunks = getenv("UB_MARCH_PAIR_MIN_CHUNKS") ? atoi(getenv("UB_MARCH_PAIR_MIN_CHUNKS")) : 2;
-  const bool pair = pair_enabled && (P.tiles_w % 2 == 0) && P.n_chunks_total >= pair_min_chunks;
+  // CTA pairs (cta_group::2) whenever the w tiles pair up and a plane has >= 2 K chunks (a plane must be long enough to
+  // amortise the cross-CTA barrier traffic: measured on B200 at 8x128^3, 1 K chunk 805 vs 1200 TFLOP/s single-CTA,
+  // 2 chunks 1374 vs 1330, 3 chunks 1576 vs 1360)
+  const bool pair = (P.tiles_w % 2 == 0) && P.n_chunks_total >= 2;
   const int wbytes = P.n_chunks_total * 9 * (pair ? kMarchWTileBytes / 2 : kMarchWTileBytes);
   const int misc = 8 * 48 + 64 + (kMarchEpiWarps * 2 * 32 + 32 + 128) * 4 + 64 + 1024;
   P.nsa = (220 * 1024 - wbytes - misc) / kMarchPlaneBytes;
@@ -529,12 +480,6 @@ static int launch_march(const void* src0, int c0p, const void* src1, int c1p, in
   if (int e = opt_in_smem(opt[variant][pair ? 1 : 0], (const void*)fn, "igemm_march")) return e;
   const unsigned grid = (unsigned)(n * P.tiles_h * P.tiles_w * P.nseg);
   const unsigned threads = tf ? kMarchThreadsTf : kMarchThreads2;
-  // two MMA-issuing warps on alternating planes in every single-CTA launch (one-chunk 32 -> 32 forward 0.875 -> 0.71 ms,
-  // its dgrad 0.85 -> 0.70, 24 -> 32 0.85 -> 0.68; three chunks without CTA pairs 2.18 -> 2.05: profiles/r02j_march_mma2.txt);
-  // UB_MARCH_MMA2=n: only layers with <= n chunks, 0: one issuer
-  static const int march_mma2 = getenv("UB_MARCH_MMA2") ? atoi(getenv("UB_MARCH_MMA2")) : 3;
-  static const bool pair_mma2 = getenv("UB_MARCH_PAIR_MMA2") && atoi(getenv("UB_MARCH_PAIR_MMA2")) != 0;   // under test
-  P.mma2 = (!tf && (!pair || pair_mma2) && march_mma2 && P.n_chunks_total <= march_mma2) ? 1 : 0;
   if (pair) {
     // cluster of two CTAs along x: blocks (2k, 2k+1) take the w tiles (2j, 2j+1) of one column pair
     cudaLaunchConfig_t cfg;
@@ -571,10 +516,9 @@ static inline int k4_shift(int k) { return k >> 1; }
 // tile (256 -> 256 @16^3 0.103 -> 0.124), except at the 8^3 level, where they double the number of tiles of an
 // underfilled grid (512 -> 512 @8^3 0.177 -> 0.120).
 static int planes_per_tile(int depth, int nt_max, int n_ntiles) {
-  static const bool td2 = !(getenv("UB_TD2") && atoi(getenv("UB_TD2")) == 0);
   int td = depth < 4 ? depth : 4;
   const int cols = (nt_max + 31) / 32 * 32;
-  if (td2 && td == 4 && 2 * 4 * cols > 512 && 2 * 2 * cols <= 512 && (n_ntiles == 1 || depth <= 8)) td = 2;
+  if (td == 4 && 2 * 4 * cols > 512 && 2 * 2 * cols <= 512 && (n_ntiles == 1 || depth <= 8)) td = 2;
   return td;
 }
 
@@ -629,9 +573,8 @@ extern "C" int ub_conv_fwd(const ub_conv_desc* d, const void* src0, const void* 
   IgemmPlan pl;
   memset(&pl, 0, sizeof(pl));
   IgemmParams& P = pl.P;
-  P.kc = d->c1p == 0 ? chunk_channels(d->kind, d->c0p, 0) : 32;
-  P.n_chunks_src0 = d->c0p / P.kc;
-  P.n_chunks_total = ktot / P.kc;
+  P.n_chunks_src0 = d->c0p / kIgemmKc;
+  P.n_chunks_total = ktot / kIgemmKc;
   P.w_rows_per_block = d->cop;
   P.Nb = d->n;
   P.bias = bias;
@@ -647,8 +590,7 @@ extern "C" int ub_conv_fwd(const ub_conv_desc* d, const void* src0, const void* 
   P.fold_nd = 3;
   P.fold_row_step = nt_max;
   P.b_block_rows = P.kd_fold ? 3 * d->cop : d->cop;
-  merged_weight_boxes(P, nt_max);
-  if (int e = make_w_map(&P.tm_w, w_packed, ktot, (long long)ntaps * d->cop, P.kc, P.b_boxes ? P.b_box_rows : nt_max)) return e;
+  if (int e = make_w_map(&P.tm_w, w_packed, ktot, (long long)ntaps * d->cop, kIgemmKc, nt_max)) return e;
 
   if (d->kind == UB_CONV_K3S1P1 || d->kind == UB_CONV_K1) {
     const int k = d->kind == UB_CONV_K3S1P1 ? 3 : 1;
@@ -740,8 +682,7 @@ extern "C" int ub_conv_fwd(const ub_conv_desc* d, const void* src0, const void* 
   P.out_s = 2;
   P.taps[0] = IgemmTap{0, 0, 0, 0};
   if (stats_partial) return fail(-1, "statistics are not produced by the transposed conv forward");
-  static const bool dc_pair = !(getenv("UB_DECONV_PAIR") && atoi(getenv("UB_DECONV_PAIR")) == 0);
-  if (dc_pair && d->cop == 64) {
+  if (d->cop == 64) {
     // 64 output channels: the sub-positions (pd, ph, 0) and (pd, ph, 1) share ONE N tile of 128 columns -- their
     // weight blocks are adjacent in the [sub-position][co][ci] pack and their voxels (2w, 2w+1) adjacent in the
     // output, so columns [64, 128) go to the same tensor one voxel further (the two-destination store of the
@@ -760,8 +701,8 @@ extern "C" int ub_conv_fwd(const ub_conv_desc* d, const void* src0, const void* 
       T.wblock_add = 2 * sp2;
       T.out_p[0] = 0; T.out_p[1] = sp2 & 1; T.out_p[2] = (sp2 >> 1) & 1;
     }
-    if (int e = make_w_map(&P.tm_w, w_packed, ktot, (long long)ntaps * d->cop, P.kc, 128)) return e;
-    if (int e = make_act_map(&P.tm_src[0], src0, d->c0p, d->w, d->h, d->d, d->n, P.kc, P.bw, P.bh, 1, plane_box(P))) return e;
+    if (int e = make_w_map(&P.tm_w, w_packed, ktot, (long long)ntaps * d->cop, kIgemmKc, 128)) return e;
+    if (int e = make_act_map(&P.tm_src[0], src0, d->c0p, d->w, d->h, d->d, d->n, kIgemmKc, P.bw, P.bh, 1, plane_box(P))) return e;
     if (int e = finish_plan(&pl, 128)) return e;
     return launch_igemm(pl, st);
   }
@@ -778,7 +719,7 @@ extern "C" int ub_conv_fwd(const ub_conv_desc* d, const void* src0, const void* 
       }
     P.n_ntiles = base_tiles * 8;
   }
-  if (int e = make_act_map(&P.tm_src[0], src0, d->c0p, d->w, d->h, d->d, d->n, P.kc, P.bw, P.bh, 1, plane_box(P))) return e;
+  if (int e = make_act_map(&P.tm_src[0], src0, d->c0p, d->w, d->h, d->d, d->n, kIgemmKc, P.bw, P.bh, 1, plane_box(P))) return e;
   if (int e = finish_plan(&pl, nt_max)) return e;
   return launch_igemm(pl, st);
 }
@@ -815,9 +756,8 @@ extern "C" int ub_conv_dgrad_fused(const ub_conv_desc* d, const void* dy, const 
   IgemmPlan pl;
   memset(&pl, 0, sizeof(pl));
   IgemmParams& P = pl.P;
-  P.kc = chunk_channels(d->kind, d->cop, 1);
-  P.n_chunks_src0 = d->cop / P.kc;
-  P.n_chunks_total = d->cop / P.kc;
+  P.n_chunks_src0 = d->cop / kIgemmKc;
+  P.n_chunks_total = d->cop / kIgemmKc;
   P.w_rows_per_block = ncols;
   P.Nb = d->n;
   P.oD = d->d; P.oH = d->h; P.oW = d->w;
@@ -831,8 +771,7 @@ extern "C" int ub_conv_dgrad_fused(const ub_conv_desc* d, const void* dy, const 
   P.fold_nd = 3;
   P.fold_row_step = nt_max;
   P.b_block_rows = P.kd_fold ? 3 * ncols : ncols;
-  merged_weight_boxes(P, nt_max);
-  if (int e = make_w_map(&P.tm_w, w_packed_dgrad, d->cop, (long long)ntaps * ncols, P.kc, P.b_boxes ? P.b_box_rows : nt_max)) return e;
+  if (int e = make_w_map(&P.tm_w, w_packed_dgrad, d->cop, (long long)ntaps * ncols, kIgemmKc, nt_max)) return e;
   bool uniform = true;
   for (int i = 0; i < P.n_ntiles; ++i) uniform = uniform && P.ntile[i].nt == nt_max;
   if (!uniform) return fail(-2, "dgrad N tiles of unequal width are not supported (c0p=%d c1p=%d)", d->c0p, d->c1p);
@@ -864,8 +803,7 @@ extern "C" int ub_conv_dgrad_fused(const ub_conv_desc* d, const void* dy, const 
     // class). With nt = 32 (stem, d2) the unfolded launches are bound by the MMA thread's instruction issue
     // (profiles/r02f_stem_fwd_ncu_summary.txt); folding halves the number of UMMAs. The sd = 0 tap block lies 32 taps
     // BEHIND the sd = 1 block in the [tap][cin][cop] pack (kd = 3 - 2 sd or 2 - 2 sd).
-    static const bool k4_fold = !(getenv("UB_K4_DGRAD_FOLD") && atoi(getenv("UB_K4_DGRAD_FOLD")) == 0);
-    const bool fold = k4_fold && P.n_ntiles == 1 && nt_max <= 128 && od >= 2;
+    const bool fold = P.n_ntiles == 1 && nt_max <= 128 && od >= 2;
     if (fold) {
       P.kd_fold = 2;
       P.fold_nd = 2;
@@ -910,12 +848,10 @@ extern "C" int ub_conv_dgrad_fused(const ub_conv_desc* d, const void* dy, const 
   // UB_DECONV_K2S2 dgrad: gather the 8 fine sub-positions (parity tiles of dy, element stride 2)
   // Two output planes per tile: the stage holds the 8 parity tiles of every plane (64 KB per plane and 32-channel
   // chunk), which leaves room for ONE stage (profiles/r02h_deconv_dgrad_ncu_summary.txt: 4 TB/s, tensor pipe 10 %,
-  // nothing near a roof). One-plane tiles with two or three stages (UB_DC_DGRAD_TD=1) are SLOWER on every level
-  // (64 -> 64 @64^3 0.61 -> 0.79 ms, profiles/r02i_wgrad_split_ab.txt): the launch is bound by the number of
-  // element-strided TMA boxes, not by exposed load latency.
-  static const int dc_td = getenv("UB_DC_DGRAD_TD") ? atoi(getenv("UB_DC_DGRAD_TD")) : 2;
-  P.td = d->d < dc_td ? d->d : dc_td;
-  if (P.kc == 64) P.td = 1;      // 8 parity tiles x 16 KB per plane: one plane per stage
+  // nothing near a roof). One-plane tiles with two or three stages were measured SLOWER on every level (64 -> 64 @64^3
+  // 0.61 -> 0.79 ms, profiles/r02i_wgrad_split_ab.txt; removed): the launch is bound by the number of element-strided
+  // TMA boxes, not by exposed load latency.
+  P.td = d->d < 2 ? d->d : 2;
   P.Do = d->d; P.Ho = d->h; P.Wo = d->w;
   P.n_atiles = 8; P.bw = 8; P.bh = 16; P.n_in_planes = P.td; P.in_stride = 2;
   P.ntaps = 8;
@@ -926,7 +862,7 @@ extern "C" int ub_conv_dgrad_fused(const ub_conv_desc* d, const void* dy, const 
         P.atile_off[at][0] = k; P.atile_off[at][1] = j; P.atile_off[at][2] = i;
         P.taps[at] = IgemmTap{(uint16_t)at, 0, 0, (uint16_t)at};
       }
-  if (int e = make_act_map(&P.tm_src[0], dy, d->cop, ow, oh, od, d->n, P.kc, P.bw, P.bh, 2, plane_box(P))) return e;
+  if (int e = make_act_map(&P.tm_src[0], dy, d->cop, ow, oh, od, d->n, kIgemmKc, P.bw, P.bh, 2, plane_box(P))) return e;
   if (int e = finish_plan(&pl, nt_max)) return e;
   return launch_igemm(pl, st);
 }
@@ -1006,9 +942,9 @@ static int plan_wgrad(const ub_conv_desc* d, WgradPlan* pl) {
   P.tiles_h = cdiv(P.Ht, 16);
   P.x_stage_bytes = align_up(P.bh * P.bw * 64, 1024);
   P.dy_stage_bytes = 128 * P.nt * 2;
-  static const bool dc_mode = !(getenv("UB_DC_WGRAD_MODE") && atoi(getenv("UB_DC_WGRAD_MODE")) == 0);
-  if (dc_mode && d->kind == UB_DECONV_K2S2 && d->c1p == 0) {
-    // chunks on the M atoms, sub-positions side by side in N (igemm_wgrad.cuh, "dc mode")
+  if (d->kind == UB_DECONV_K2S2) {
+    // chunks on the M atoms, sub-positions side by side in N (igemm_wgrad.cuh, "dc mode"); one CTA per (chunk,
+    // sub-position) measured slower (profiles/r02i_dc_wgrad_ab.txt), removed
     P.chunk_atoms = P.n_chunks_total < 4 ? P.n_chunks_total : 4;
     P.var_boxes = 256 / P.nt >= 8 ? 8 : (256 / P.nt >= 4 ? 4 : (256 / P.nt >= 2 ? 2 : 1));
     P.x_stage_bytes = P.chunk_atoms * P.bh * P.bw * 64;      // 8 KB tiles, already 1024-aligned
@@ -1025,25 +961,21 @@ static int plan_wgrad(const ub_conv_desc* d, WgradPlan* pl) {
                                   : P.n_chunks_total * P.n_variants * P.n_cotiles;
   // Splits of the voxel range per (chunk, variant, co tile) item. The CTAs are not persistent, so the grid must fill
   // whole waves of the CTAs an SM can hold (shared memory and TMEM columns decide: one or two, three for the narrow
-  // layers). The old rule, cdiv(2 * 148, items), put 304 CTAs on 296 slots for the 64 -> 64 transposed conv: a second
-  // wave of 8 CTAs, SMs active 57 % of the launch (profiles/r02h_deconv_wgrad_ncu_summary.txt). Now: the split count
-  // that minimises waves x tiles-per-split, up to four waves' worth; UB_WGRAD_SPLIT_OLD=1 restores the old rule.
-  static const bool old_rule = getenv("UB_WGRAD_SPLIT_OLD") && atoi(getenv("UB_WGRAD_SPLIT_OLD")) != 0;
-  long long nsplit = cdiv(2 * 148, items);
-  if (!old_rule) {
-    int occ = (228 * 1024) / (pl->smem + 1024);
-    if (occ > 512 / P.tmem_cols) occ = 512 / P.tmem_cols;
-    if (occ > 4) occ = 4;
-    if (occ < 1) occ = 1;
-    const long long cap = (long long)occ * sm_count();
-    long long best = 1, best_cost = -1;
-    const long long ns_max = cdiv(4 * cap, items) < total_tiles ? cdiv(4 * cap, items) : total_tiles;
-    for (long long ns = 1; ns <= ns_max; ++ns) {
-      // time ~ waves x (tiles per split + a fixed per-CTA cost: pipeline fill, TMEM read-out, partial record)
-      const long long cost = cdiv(items * ns, cap) * (cdiv(total_tiles, ns) + 32);
-      if (best_cost < 0 || cost < best_cost) { best = ns; best_cost = cost; }
-    }
-    nsplit = best;
+  // layers). The earlier rule, cdiv(2 * 148, items), put 304 CTAs on 296 slots for the 64 -> 64 transposed conv: a
+  // second wave of 8 CTAs, SMs active 57 % of the launch (profiles/r02h_deconv_wgrad_ncu_summary.txt; measured against
+  // this one in profiles/r02i_wgrad_split_ab.txt, removed). Now: the split count that minimises waves x tiles-per-split,
+  // up to four waves' worth.
+  int occ = (228 * 1024) / (pl->smem + 1024);
+  if (occ > 512 / P.tmem_cols) occ = 512 / P.tmem_cols;
+  if (occ > 4) occ = 4;
+  if (occ < 1) occ = 1;
+  const long long cap = (long long)occ * sm_count();
+  long long nsplit = 1, best_cost = -1;
+  const long long ns_max = cdiv(4 * cap, items) < total_tiles ? cdiv(4 * cap, items) : total_tiles;
+  for (long long ns = 1; ns <= ns_max; ++ns) {
+    // time ~ waves x (tiles per split + a fixed per-CTA cost: pipeline fill, TMEM read-out, partial record)
+    const long long cost = cdiv(items * ns, cap) * (cdiv(total_tiles, ns) + 32);
+    if (best_cost < 0 || cost < best_cost) { nsplit = ns; best_cost = cost; }
   }
   if (nsplit > total_tiles) nsplit = total_tiles;
   if (nsplit < 1) nsplit = 1;
@@ -1066,18 +998,17 @@ static int wgrad_march_splits(const ub_conv_desc* d) {
 }
 
 // split-K reduction of the weight-gradient partial records into the torch layout: many splits of a small output ->
-// the 8-lanes-per-output kernel; large outputs -> the tiled transpose; the rest -> one thread per output
-// (UB_WGRAD_REDUCE_OLD=1: never the tiled kernel, for A/B).
+// the 8-lanes-per-output kernel; large outputs -> the tiled transpose (measured against one thread per output in
+// profiles/r02i_reduce_pack_ab.txt); the rest -> one thread per output.
 static void launch_wgrad_reduce(const float* partial, float* dw, const WgradReduceArgs& R, cudaStream_t st) {
   const long long per_split = (long long)R.ntap * R.ci_total * R.co_total;
-  const bool old_reduce = getenv("UB_WGRAD_REDUCE_OLD") && atoi(getenv("UB_WGRAD_REDUCE_OLD")) != 0;
   int dst_ntaps = 0;
   bool unit_taps = R.dst_tap_stride == 1;
   for (int i = 0; i < R.ntap && i < 64; ++i)
     if (R.tapmap[i] + 1 > dst_ntaps) dst_ntaps = R.tapmap[i] + 1;
   if (per_split <= 65536 && R.nsplit >= 32)
     wgrad_reduce_wide_kernel<<<(unsigned)((per_split * 8 + 255) / 256), 256, 0, st>>>(partial, dw, R);
-  else if (old_reduce || !unit_taps || dst_ntaps < 1 || dst_ntaps > 64 || R.ntap > 64 ||
+  else if (!unit_taps || dst_ntaps < 1 || dst_ntaps > 64 || R.ntap > 64 ||
            R.ci_total * cdiv(R.co_total, kRedTileCols) < 512)
     wgrad_reduce_kernel<<<(unsigned)((per_split + 255) / 256), 256, 0, st>>>(partial, dw, R);
   else
@@ -1142,8 +1073,6 @@ extern "C" int ub_conv_wgrad(const ub_conv_desc* d, const void* src0, const void
     static SmemOptIn wopt[3];
     const int wv = stem ? 1 : (src0_act ? 2 : 0);
     if (int e = opt_in_smem(wopt[wv], (const void*)wfns[wv], "wgrad_march")) return e;
-    static const bool wm_mma2 = !(getenv("UB_WGRAD_MMA2") && atoi(getenv("UB_WGRAD_MMA2")) == 0);
-    M.mma2 = wm_mma2 ? 1 : 0;
     const int nsplit = wgrad_march_splits(d);
     const int smem = kWmXStages * kWmXBytes + (kWmYSlots + kt - 1) * kWmYBytes + 8 * 32 + 64 + 1024;
     const dim3 grid((unsigned)nsplit, (unsigned)(M.n_chunks_total * M.n_cotiles * (stem ? 8 : 1)));

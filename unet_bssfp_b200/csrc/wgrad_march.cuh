@@ -38,7 +38,6 @@ struct WgradMarchParams {
   // deferred activation: the four epilogue warps, idle until the end, rewrite every X halo plane of chunk 0 in
   // shared memory (deferred_tile.cuh) before the MMA thread reads it.
   NormActArgs tf;
-  int mma2;                 // two MMA-issuing warps: warp 5 takes the kh groups [0, KT - 1), warp 7 the last one (KT = 2: one each)
 };
 
 constexpr int kWmXStages = 4, kWmXBytes = 12288;
@@ -46,10 +45,11 @@ constexpr int kWmYSlots = 8, kWmYBytes = 8192;   // + KT-1 mirror slots
 
 // Warps 0-3 epilogue (kTf: operand transform first), 4 TMA producer of the X planes, 5 MMA issuer, 6 TMA producer of the
 // dY planes (two producer threads: the stem form has 16 UMMAs of 48 cycles per plane against two to three TMA boxes),
-// 7 second MMA issuer (mma2). The two issuers own DIFFERENT kh accumulators -- nothing orders them against each other,
-// unlike two threads accumulating into one accumulator -- and walk the same barriers; one's per-plane hand-off (waits,
-// fence, commits) runs while the other's UMMAs are in the pipe (the marching kernels spend ~450 cycles per plane on it
-// beside UMMAs that run at their isolated rate, profiles/r02j_march_mma_ablation.txt).
+// 7 second MMA issuer: warp 5 takes the kh groups [0, KT - 1), warp 7 the last one (KT = 2: one each). The two issuers own
+// DIFFERENT kh accumulators -- nothing orders them against each other, unlike two threads accumulating into one
+// accumulator -- and walk the same barriers; one's per-plane hand-off (waits, fence, commits) runs while the other's UMMAs
+// are in the pipe (the marching kernels spend ~450 cycles per plane on it beside UMMAs that run at their isolated rate,
+// profiles/r02j_march_mma_ablation.txt). One issuer measured slower (profiles/r02j_wgrad_mma2.txt), removed.
 constexpr int kWgradMarchThreads = kIgemmThreads + 64;
 template <int KT, bool kTf>
 __global__ void __launch_bounds__(kWgradMarchThreads, 1)
@@ -87,12 +87,12 @@ wgrad_march_kernel(const __grid_constant__ WgradMarchParams P) {
   int i_end = i_begin + per; if (i_end > items) i_end = items;
 
   if (threadIdx.x == 0) {
-    const uint32_t nmma = P.mma2 ? 2u : 1u;      // every issuer commits the stage / slot / accumulator barriers
+    // both issuers commit the stage / slot / accumulator barriers
     for (int i = 0; i < kWmXStages; ++i) {
-      mbar_init(x_full + 8 * i, 1); mbar_init(x_empty + 8 * i, nmma); mbar_init(x_ready + 8 * i, 1);
+      mbar_init(x_full + 8 * i, 1); mbar_init(x_empty + 8 * i, 2); mbar_init(x_ready + 8 * i, 1);
     }
-    for (int i = 0; i < kWmYSlots; ++i) { mbar_init(y_full + 8 * i, 1); mbar_init(y_empty + 8 * i, nmma); }
-    mbar_init(acc_full, nmma);
+    for (int i = 0; i < kWmYSlots; ++i) { mbar_init(y_full + 8 * i, 1); mbar_init(y_empty + 8 * i, 2); }
+    mbar_init(acc_full, 2);
     fence_mbar_init();
   }
   if (warp == 4 && lane == 0) tma_prefetch_desc(&P.tm_x[s1 ? 1 : 0]);
@@ -156,10 +156,8 @@ wgrad_march_kernel(const __grid_constant__ WgradMarchParams P) {
     __syncwarp();
   } else if (warp == 5 || warp == 7) {
     // =========================== MMA issuer(s) ===========================
-    const int kh_begin = (P.mma2 && warp == 7) ? KT - 1 : 0;
-    const int kh_end = (P.mma2 && warp == 5) ? KT - 1 : KT;
-    const bool active = warp == 5 || P.mma2;          // without mma2 warp 7 has nothing to do
-    const int it_end = active ? i_end : i_begin;
+    const int kh_begin = warp == 7 ? KT - 1 : 0;
+    const int kh_end = warp == 5 ? KT - 1 : KT;
     const uint32_t idesc = make_idesc_bf16(128, NN, 1, 1);
     const uint64_t a_desc0 = make_smem_desc(0, /*lbo: next kw atom = next halo row*/ 64, /*sbo: next h row*/ BW * 64, SWZ_64B);
     const uint64_t b_desc0 = make_smem_desc(0, /*lbo: next dY plane*/ kWmYBytes, /*sbo: next 8 voxel rows*/ 8 * 64, SWZ_64B);
@@ -169,7 +167,7 @@ wgrad_march_kernel(const __grid_constant__ WgradMarchParams P) {
     int xs = 0; uint32_t xp = 0;
     int ys = 0; uint32_t yp = 0;       // slot / phase of the OLDEST of the KT live dY planes
     uint32_t first = 1;
-    for (int it = i_begin; it < it_end; ++it) {
+    for (int it = i_begin; it < i_end; ++it) {
       const int seg = it % P.nseg;
       const int d0 = seg * P.seg_len;
       int d1 = d0 + P.seg_len; if (d1 > P.D) d1 = P.D;
@@ -218,7 +216,7 @@ wgrad_march_kernel(const __grid_constant__ WgradMarchParams P) {
         if (ys >= kWmYSlots) { ys -= kWmYSlots; yp ^= 1; }
       }
     }
-    if (leader && active) umma_commit(acc_full);
+    if (leader) umma_commit(acc_full);
     __syncwarp();
   } else {
     if (tf_cta) {
