@@ -149,7 +149,7 @@ int ub_pack_ncdhw_s2d(const void* a, int a_bf16, int ca, const float* b, int cb,
  * reads its input this way through UB_CONV_K4S2P1_S2D instead of strided TMA boxes. */
 int ub_to_s2d(const void* src, int n, int d, int h, int w, int cp, void* dst, void* stream);
 /* Sliding-window inference (ref:model.py:315-333, ref:data_module.py:168-183; torchio==0.19.6
- * GridSampler / GridAggregator with patch_overlap 0). ub_pack_patches gathers n (<= 64) d x h x w patches of
+ * GridSampler / GridAggregator, any patch_overlap). ub_pack_patches gathers n (<= 64) d x h x w patches of
  * an NCDHW fp32 volume into one NDHWC bf16 batch: patch i starts at element offsets[i] (HOST array) of `a`,
  * its element (c,z,y,x) is at + c*stride_c + z*stride_d + y*stride_h + x. ub_unpack_patch writes channels
  * [c_begin, c_begin+c) of batch sample `sample` into the volume region at dst + dst_offset (same
@@ -161,6 +161,17 @@ int ub_unpack_patch(const void* src, int cp, int c_begin, int c, int sample, int
 /* the same aggregation for an NCDHW fp32 patch [c][d][h][w] (the output of ub_conv1x1_to_ncdhw) */
 int ub_paste_patch(const float* src, int c, int d, int h, int w, float* dst, long long dst_offset,
                    long long stride_c, long long stride_d, long long stride_h, void* stream);
+/* GridAggregator.add_batch for one batch of n (<= 64) NCDHW fp32 patches src [n][c <= 8][pd][ph][pw], in sampler
+ * order, in ONE launch. origins (HOST, [n][3]): patch origins (z, y, x) in the volume; boxes (HOST, [n][6] z0 y0 x0
+ * z1 y1 x1, half-open, inside the patch; NULL = the whole patch): the region each patch writes. out [c][d][h][w] and
+ * weight [d][h][w] are contiguous fp32 volumes. mode 0 'crop': the last patch whose box holds a voxel is assigned
+ * (weight unused); mode 1 'average': out += p, weight += 1; mode 2 'hann': out += p * w, weight += w with
+ * w = (wz[z] * wy[y]) * wx[x] read from window (DEVICE, pd + ph + pw floats: wz, wy, wx). Each voxel sums its
+ * patches in order with separately rounded fp32 multiplies and adds, so launches in sampler order reproduce
+ * torchio's tensors bit for bit. ub_blend_finish: out /= weight (every channel) after the last batch. */
+int ub_blend_patches(const float* src, int n, int c, int pd, int ph, int pw, const int* origins, const int* boxes,
+                     int mode, const float* window, float* out, float* weight, int d, int h, int w, void* stream);
+int ub_blend_finish(float* out, const float* weight, int c, long long voxels, void* stream);
 /* NDHWC bf16 (cp channels) -> NCDHW fp32, channels [c_begin, c_begin + c) */
 int ub_unpack_ncdhw(const void* src, int cp, int c_begin, int c, int n, long long voxels, float* out,
                     void* stream);

@@ -81,6 +81,9 @@ SIGNATURES = {
     "ub_pack_patches": (_I, [_P, _I, _I, C.POINTER(C.c_longlong), _I, _I, _I, _LL, _LL, _LL, _I, _P, _P]),
     "ub_unpack_patch": (_I, [_P, _I, _I, _I, _I, _I, _I, _I, _P, _LL, _LL, _LL, _LL, _P]),
     "ub_paste_patch": (_I, [_P, _I, _I, _I, _I, _P, _LL, _LL, _LL, _LL, _P]),
+    "ub_blend_patches": (_I, [_P, _I, _I, _I, _I, _I, C.POINTER(C.c_int), C.POINTER(C.c_int), _I, _P, _P, _P, _I, _I,
+                              _I, _P]),
+    "ub_blend_finish": (_I, [_P, _P, _I, _LL, _P]),
     "ub_unpack_ncdhw": (_I, [_P, _I, _I, _I, _I, _LL, _P, _P]),
     "ub_conv1x1_workspace_bytes": (_LL, []),
     "ub_conv1x1_to_ncdhw": (_I, [_P, _I, _P, _I, _P, _I, _I, _LL, _P, _P, _AP, _P]),

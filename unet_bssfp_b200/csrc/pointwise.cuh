@@ -467,6 +467,95 @@ __global__ void paste_patch_kernel(const float* __restrict__ src, float* __restr
   for (int k = 0; k < c; ++k) d[(size_t)k * G.stride_c] = __ldcs(src + (size_t)k * V + v);
 }
 
+// Overlapping sliding-window aggregation (torchio 0.19.6 GridAggregator.add_batch): up to kMaxPatchBatch NCDHW fp32
+// patches [n][c][pd][ph][pw], in sampler order, into an NCDHW fp32 volume. One thread per voxel of the batch's
+// bounding box (x fastest) tests the patches' boxes in order:
+//   kBlendCrop     the last patch whose box (its crop box) holds the voxel is assigned: "the later patch wins";
+//   kBlendAverage  out += p and weight += 1 for every covering patch;
+//   kBlendHann     w = (wz * wy) * wx from the window vectors, out += p * w and weight += w.
+// The accumulating modes keep the voxel's numerator and weight in registers across the batch and load / store them
+// once, so each voxel sees its additions in sampler order, across launches too. __fmul_rn / __fadd_rn keep nvcc
+// from contracting num + p * w into an FMA: the sums are the ones torch computes, bit for bit.
+enum BlendMode { kBlendCrop = 0, kBlendAverage = 1, kBlendHann = 2 };
+constexpr int kMaxBlendChannels = 8;
+struct BlendGeom {
+  int org[kMaxPatchBatch][3];             // patch origin (z, y, x) in the volume
+  int box[kMaxPatchBatch][6];             // volume region the patch writes: z0, y0, x0, z1, y1, x1 (half-open)
+  int n, c, pd, ph, pw;
+  int b0[3], bh, bw;                      // bounding box of the batch's boxes: origin and its two inner extents
+  int H, W;                               // volume [c][D][H][W] and weight [D][H][W], both contiguous
+  long long V;                            // D * H * W
+};
+template <int MODE>
+__global__ void __launch_bounds__(256)
+blend_patches_kernel(const float* __restrict__ src, float* __restrict__ out, float* __restrict__ weight,
+                     const float* __restrict__ window /* wz[pd], wy[ph], wx[pw] */, const __grid_constant__ BlendGeom G,
+                     uint32_t voxels) {
+  const uint32_t v = blockIdx.x * 256u + threadIdx.x;
+  if (v >= voxels) return;
+  const uint32_t t = v / (uint32_t)G.bw;
+  const int x = G.b0[2] + (int)(v - t * (uint32_t)G.bw);
+  const int y = G.b0[1] + (int)(t % (uint32_t)G.bh);
+  const int z = G.b0[0] + (int)(t / (uint32_t)G.bh);
+  const size_t PV = (size_t)G.pd * G.ph * G.pw;
+  const size_t vox = ((size_t)z * G.H + y) * G.W + x;
+  float* o = out + vox;
+  auto local = [&](int j) {                // element (0, lz, ly, lx) of patch j
+    return ((size_t)j * G.c * G.pd + (z - G.org[j][0])) * G.ph * G.pw + (size_t)(y - G.org[j][1]) * G.pw + (x - G.org[j][2]);
+  };
+  auto covers = [&](int j) {
+    return z >= G.box[j][0] && y >= G.box[j][1] && x >= G.box[j][2] && z < G.box[j][3] && y < G.box[j][4] && x < G.box[j][5];
+  };
+  if (MODE == kBlendCrop) {
+    int last = -1;
+    for (int j = 0; j < G.n; ++j)
+      if (covers(j)) last = j;
+    if (last < 0) return;
+    const float* s = src + local(last);
+    for (int k = 0; k < G.c; ++k) o[(size_t)k * G.V] = __ldcs(s + (size_t)k * PV);
+    return;
+  }
+  float num[kMaxBlendChannels];
+  float den = 0.f;
+  bool any = false;
+  for (int j = 0; j < G.n; ++j) {
+    if (!covers(j)) continue;
+    if (!any) {
+      any = true;
+      den = weight[vox];
+#pragma unroll
+      for (int k = 0; k < kMaxBlendChannels; ++k)
+        if (k < G.c) num[k] = o[(size_t)k * G.V];
+    }
+    const float* s = src + local(j);
+    float w = 1.f;
+    if (MODE == kBlendHann)
+      w = __fmul_rn(__fmul_rn(window[z - G.org[j][0]], window[G.pd + (y - G.org[j][1])]),
+                    window[G.pd + G.ph + (x - G.org[j][2])]);
+#pragma unroll
+    for (int k = 0; k < kMaxBlendChannels; ++k) {
+      if (k >= G.c) break;
+      const float p = __ldcs(s + (size_t)k * PV);
+      num[k] = __fadd_rn(num[k], MODE == kBlendHann ? __fmul_rn(p, w) : p);
+    }
+    den = __fadd_rn(den, w);
+  }
+  if (!any) return;
+  weight[vox] = den;
+#pragma unroll
+  for (int k = 0; k < kMaxBlendChannels; ++k)
+    if (k < G.c) o[(size_t)k * G.V] = num[k];
+}
+
+// out / weight after the last batch of an accumulating blend: the true_divide of GridAggregator.get_output_tensor.
+__global__ void __launch_bounds__(256)
+blend_finish_kernel(float* __restrict__ out, const float* __restrict__ weight, int c, uint32_t voxels) {
+  const uint32_t v = blockIdx.x * 256u + threadIdx.x;
+  if (v >= voxels) return;
+  const float w = weight[v];
+  for (int k = 0; k < c; ++k) out[(size_t)k * voxels + v] = __fdiv_rn(out[(size_t)k * voxels + v], w);
+}
+
 // channels [c_begin, c_begin + c) of an NDHWC bf16 tensor -> NCDHW fp32
 __global__ void unpack_ncdhw_kernel(const __nv_bfloat16* __restrict__ src, float* __restrict__ dst, int cp,
                                     int c_begin, int c, long long V, long long total) {

@@ -1237,6 +1237,53 @@ extern "C" int ub_paste_patch(const float* src, int c, int d, int h, int w, floa
   return 0;
 }
 
+extern "C" int ub_blend_patches(const float* src, int n, int c, int pd, int ph, int pw, const int* origins,
+                                const int* boxes, int mode, const float* window, float* out, float* weight, int d,
+                                int h, int w, void* stream) {
+  if (!src || !out || !origins || n <= 0 || c <= 0 || pd <= 0 || ph <= 0 || pw <= 0 || d <= 0 || h <= 0 || w <= 0)
+    return fail(-1, "bad arguments to ub_blend_patches");
+  if (n > kMaxPatchBatch) return fail(-1, "ub_blend_patches: at most %d patches per call", kMaxPatchBatch);
+  if (c > kMaxBlendChannels) return fail(-1, "ub_blend_patches: at most %d channels, got %d", kMaxBlendChannels, c);
+  if (mode != kBlendCrop && mode != kBlendAverage && mode != kBlendHann) return fail(-1, "ub_blend_patches: unknown mode %d", mode);
+  if (mode != kBlendCrop && !weight) return fail(-1, "ub_blend_patches: the accumulating modes need the weight volume");
+  if (mode == kBlendHann && !window) return fail(-1, "ub_blend_patches: hann mode needs the window vectors");
+  BlendGeom G;
+  memset(&G, 0, sizeof(G));
+  G.n = n; G.c = c; G.pd = pd; G.ph = ph; G.pw = pw; G.H = h; G.W = w; G.V = (long long)d * h * w;
+  const int dims[3] = {d, h, w}, p[3] = {pd, ph, pw};
+  int lo[3] = {d, h, w}, hi[3] = {0, 0, 0};
+  for (int i = 0; i < n; ++i) {
+    for (int a = 0; a < 3; ++a) {
+      const int o = origins[3 * i + a];
+      const int b0 = boxes ? boxes[6 * i + a] : o, b1 = boxes ? boxes[6 * i + 3 + a] : o + p[a];
+      if (o < 0 || o + p[a] > dims[a] || b0 < o || b1 > o + p[a] || b0 >= b1)
+        return fail(-1, "ub_blend_patches: patch %d (origin %d, box [%d, %d) on axis %d) leaves the patch or the volume", i, o, b0, b1, a);
+      G.org[i][a] = o; G.box[i][a] = b0; G.box[i][3 + a] = b1;
+      lo[a] = b0 < lo[a] ? b0 : lo[a];
+      hi[a] = b1 > hi[a] ? b1 : hi[a];
+    }
+  }
+  for (int a = 0; a < 3; ++a) G.b0[a] = lo[a];
+  G.bh = hi[1] - lo[1]; G.bw = hi[2] - lo[2];
+  const long long V = (long long)(hi[0] - lo[0]) * G.bh * G.bw;
+  if (G.V >= (1ll << 31)) return fail(-2, "ub_blend_patches: volume too large");
+  const dim3 grid((unsigned)((V + 255) / 256));
+  cudaStream_t st = (cudaStream_t)stream;
+  if (mode == kBlendCrop) blend_patches_kernel<kBlendCrop><<<grid, 256, 0, st>>>(src, out, weight, window, G, (uint32_t)V);
+  else if (mode == kBlendAverage) blend_patches_kernel<kBlendAverage><<<grid, 256, 0, st>>>(src, out, weight, window, G, (uint32_t)V);
+  else blend_patches_kernel<kBlendHann><<<grid, 256, 0, st>>>(src, out, weight, window, G, (uint32_t)V);
+  UB_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int ub_blend_finish(float* out, const float* weight, int c, long long voxels, void* stream) {
+  if (!out || !weight || c <= 0 || voxels <= 0) return fail(-1, "bad arguments to ub_blend_finish");
+  if (voxels >= (1ll << 31)) return fail(-2, "ub_blend_finish: volume too large");
+  blend_finish_kernel<<<(unsigned)((voxels + 255) / 256), 256, 0, (cudaStream_t)stream>>>(out, weight, c, (uint32_t)voxels);
+  UB_LAUNCH_CHECK();
+  return 0;
+}
+
 extern "C" int ub_unpack_ncdhw(const void* src, int cp, int c_begin, int c, int n, long long voxels, float* out,
                                void* stream) {
   if (!src || !out || c <= 0 || c_begin < 0 || c_begin + c > cp || cp % 8) return fail(-1, "bad arguments to ub_unpack_ncdhw");

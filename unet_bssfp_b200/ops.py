@@ -19,7 +19,7 @@ from ._lib import (ConvDesc, UB_PACK_F16_SRC0, UB_CONV_K1, UB_CONV_K3S1P1, UB_CO
 
 __all__ = [
     "ConvSpec", "DeferredAct", "UB_PACK_F16_SRC0", "deferred_src0_ok", "pad32", "pack_conv_weights", "pack_conv_weights_multi", "conv_fwd", "conv_dgrad", "conv_wgrad", "conv1x1_to_ncdhw", "conv1x1_from_ncdhw_bwd", "pack_ncdhw", "unpack_ncdhw",
-    "pack_patches", "unpack_patch", "paste_patch",
+    "pack_patches", "unpack_patch", "paste_patch", "blend_patches", "blend_finish",
     "norm_finalize", "bn_running_update", "norm_act_fwd", "norm_act_bwd", "maxpool_bwd", "colsum", "l1_fwd", "l1_bwd", "bce_logits",
     "scale_by", "relerr_map_reduce", "dti_scalar_maps", "denorm_to_nifti",
 ]
@@ -474,6 +474,51 @@ def paste_patch(patch: torch.Tensor, volume: torch.Tensor, origin):
         raise RuntimeError(f"patch at {origin} of size {(pd, ph, pw)} leaves the volume {(D, H, W)}")
     _lib.check(lib.ub_paste_patch(_p(patch), c, pd, ph, pw, _p(volume), z * sd + y * sh + x, sc, sd, sh, _stream()),
                "ub_paste_patch")
+
+
+BLEND_MODES = ("crop", "average", "hann")
+
+
+def blend_patches(patches: torch.Tensor, volume: torch.Tensor, origins, mode: str = "crop", boxes=None,
+                  weight: torch.Tensor | None = None, window: torch.Tensor | None = None):
+    """Aggregate a batch of NCDHW fp32 patches (n, c, pd, ph, pw), in sampler order, into the contiguous (c, D, H, W)
+    fp32 ``volume`` in one launch (torchio ``GridAggregator.add_batch``). ``origins``: (z, y, x) per patch; ``boxes``:
+    (z0, y0, x0, z1, y1, x1) volume region each patch writes (default: the whole patch). ``mode``: "crop" (the later
+    patch wins), "average" (``volume += p``, ``weight += 1``) or "hann" (``volume += p * w``, ``weight += w``,
+    ``w = (wz * wy) * wx`` from ``window`` = cat[wz, wy, wx], fp32 on the device). ``weight``: contiguous (D, H, W) fp32,
+    needed by the accumulating modes; ``blend_finish`` divides once after the last batch."""
+    _require_cuda(patches, volume, weight, window)
+    lib = _lib.load()
+    if mode not in BLEND_MODES:
+        raise ValueError(f"overlap mode must be one of {BLEND_MODES}, got {mode!r}")
+    if patches.dtype != torch.float32 or not patches.is_contiguous() or patches.dim() != 5:
+        raise RuntimeError("blend_patches reads a contiguous (n, c, pd, ph, pw) fp32 tensor")
+    if volume.dtype != torch.float32 or volume.dim() != 4 or not volume.is_contiguous():
+        raise RuntimeError("blend_patches writes into a contiguous (C, D, H, W) fp32 tensor")
+    n, c, pd, ph, pw = patches.shape
+    _, D, H, W = volume.shape
+    if volume.shape[0] != c or len(origins) != n:
+        raise RuntimeError(f"blend_patches: {n} patches of {c} channels, {len(origins)} origins, volume {tuple(volume.shape)}")
+    if mode != "crop" and (weight is None or weight.dtype != torch.float32 or tuple(weight.shape) != (D, H, W)
+                           or not weight.is_contiguous()):
+        raise RuntimeError(f"blend_patches: mode {mode!r} needs a contiguous ({D}, {H}, {W}) fp32 weight volume")
+    if mode == "hann" and (window is None or window.dtype != torch.float32 or window.numel() != pd + ph + pw):
+        raise RuntimeError(f"blend_patches: hann mode needs the {pd} + {ph} + {pw} fp32 window values")
+    orgs = (C.c_int * (3 * n))(*[v for o in origins for v in o])
+    bx = None if boxes is None else (C.c_int * (6 * n))(*[v for b in boxes for v in b])
+    _lib.check(lib.ub_blend_patches(_p(patches), n, c, pd, ph, pw, orgs, bx, BLEND_MODES.index(mode),
+                                    _p(window.contiguous()) if mode == "hann" else None, _p(volume),
+                                    _p(weight) if mode != "crop" else None, D, H, W, _stream()), "ub_blend_patches")
+
+
+def blend_finish(volume: torch.Tensor, weight: torch.Tensor):
+    """``volume /= weight`` in place over every channel: the end of an accumulating ``blend_patches`` sequence."""
+    _require_cuda(volume, weight)
+    if (volume.dtype != torch.float32 or volume.dim() != 4 or not volume.is_contiguous() or weight.dtype != torch.float32
+            or tuple(weight.shape) != tuple(volume.shape[1:]) or not weight.is_contiguous()):
+        raise RuntimeError("blend_finish: a contiguous (C, D, H, W) fp32 volume and its (D, H, W) fp32 weight")
+    _lib.check(_lib.load().ub_blend_finish(_p(volume), _p(weight), volume.shape[0], weight.numel(), _stream()),
+               "ub_blend_finish")
 
 
 def unpack_ncdhw(x: torch.Tensor, c: int, c_begin: int = 0) -> torch.Tensor:
