@@ -18,6 +18,7 @@ import torch
 from tests.conv_exact import (DECONV_K2S2, K1, K3S1P1, K4S2P1, K4S2P1_S2D, check_exact_bound, epilogue_fp32,
                               granularity, int_operand, pad_channels, ref_dgrad, ref_fwd, ref_wgrad, round_out, to_s2d,
                               weight_shape)
+from tests.step_census import run_step
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -57,45 +58,34 @@ def _label(e):
 
 def record_census(modality, batch, size):
     """Run one GanTrainer step with recording wrappers; -> sorted list of distinct Entry."""
-    import unet_bssfp_b200 as ub
-    from unet_bssfp_b200.train_step import GanTrainer
     ops = _ops()
     seen = set()
-    fwd0, dgrad0, wgrad0 = ops.conv_fwd, ops.conv_dgrad, ops.conv_wgrad
 
-    def fwd(spec, src0, src1, w_packed, bias, act=0, slope=0.0, want_stats=False):
-        assert not isinstance(src0, ops.DeferredAct), "the census records the default (materialised) operand paths"
-        seen.add(Entry("fwd", spec.kind, spec.c0, spec.c1, spec.co, spec.in_dims(src0), bool(want_stats), int(act),
-                       float(slope) if act else 0.0, src0.dtype == torch.float16, False, bias is not None))
-        return fwd0(spec, src0, src1, w_packed, bias, act=act, slope=slope, want_stats=want_stats)
+    def fwd(fwd0):
+        def wrapper(spec, src0, src1, w_packed, bias, act=0, slope=0.0, want_stats=False):
+            assert not isinstance(src0, ops.DeferredAct), "the census records the default (materialised) operand paths"
+            seen.add(Entry("fwd", spec.kind, spec.c0, spec.c1, spec.co, spec.in_dims(src0), bool(want_stats), int(act),
+                           float(slope) if act else 0.0, src0.dtype == torch.float16, False, bias is not None))
+            return fwd0(spec, src0, src1, w_packed, bias, act=act, slope=slope, want_stats=want_stats)
+        return wrapper
 
-    def dgrad(spec, dy, w_packed_dgrad, in_dhw, fuse=None):
-        seen.add(Entry("dgrad", spec.kind, spec.c0, spec.c1, spec.co, (dy.shape[0],) + tuple(in_dhw), False, 0,
-                       float(fuse.slope) if fuse is not None else 0.0, False, fuse is not None, False,
-                       float(fuse.drop_p) if fuse is not None else 0.0))
-        return dgrad0(spec, dy, w_packed_dgrad, in_dhw, fuse=fuse)
+    def dgrad(dgrad0):
+        def wrapper(spec, dy, w_packed_dgrad, in_dhw, fuse=None):
+            seen.add(Entry("dgrad", spec.kind, spec.c0, spec.c1, spec.co, (dy.shape[0],) + tuple(in_dhw), False, 0,
+                           float(fuse.slope) if fuse is not None else 0.0, False, fuse is not None, False,
+                           float(fuse.drop_p) if fuse is not None else 0.0))
+            return dgrad0(spec, dy, w_packed_dgrad, in_dhw, fuse=fuse)
+        return wrapper
 
-    def wgrad(spec, src0, src1, dy, weight_shape):
-        assert not isinstance(src0, ops.DeferredAct)
-        seen.add(Entry("wgrad", spec.kind, spec.c0, spec.c1, spec.co, spec.in_dims(src0), False, 0, 0.0, False, False,
-                       False))
-        return wgrad0(spec, src0, src1, dy, weight_shape)
+    def wgrad(wgrad0):
+        def wrapper(spec, src0, src1, dy, weight_shape):
+            assert not isinstance(src0, ops.DeferredAct)
+            seen.add(Entry("wgrad", spec.kind, spec.c0, spec.c1, spec.co, spec.in_dims(src0), False, 0, 0.0, False,
+                           False, False))
+            return wgrad0(spec, src0, src1, dy, weight_shape)
+        return wrapper
 
-    cin = 24 if modality == "bssfp" else 6
-    with pytest.MonkeyPatch.context() as mp:
-        mp.setattr(ops, "conv_fwd", fwd)
-        mp.setattr(ops, "conv_dgrad", dgrad)
-        mp.setattr(ops, "conv_wgrad", wgrad)
-        torch.manual_seed(0)
-        g, d = ub.Generator(modality).to(DEV), ub.Discriminator(modality).to(DEV)
-        tr = GanTrainer(g, d)
-        torch.manual_seed(1)
-        x = torch.rand(batch, cin, size, size, size, device=DEV)
-        y = torch.rand(batch, 6, size, size, size, device=DEV)
-        tr.step(x, y)
-        torch.cuda.synchronize()
-        del tr, g, d, x, y
-    torch.cuda.empty_cache()
+    run_step(modality, batch, size, {"conv_fwd": fwd, "conv_dgrad": dgrad, "conv_wgrad": wgrad})
     return sorted(seen, key=lambda e: (list(DIRS).index(e.dir), e.kind, e.c0, e.c1, e.co, e.dims, e.stats, e.f16, e.fuse))
 
 

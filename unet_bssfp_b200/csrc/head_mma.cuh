@@ -192,20 +192,22 @@ head_bwd_sums_mma_kernel(const float* __restrict__ dout, const __nv_bfloat16* __
     for (int grp = 0; grp < 2; ++grp) {
       const bf16x8& yraw = grp ? C.yb : C.ya;
       const unsigned long long e0 = ((unsigned long long)n * V + va + 8u * grp) * 32ull + tig * 8;
-      const bf16x8 a8 = K.apply(yraw, e0);
+      uint32_t keep[4];
+      const bf16x8 a8 = K.apply(yraw, e0, nullptr, keep);
       const uint32_t* aw = reinterpret_cast<const uint32_t*>(&a8);
 #pragma unroll
       for (int r = 0; r < 4; ++r) (grp ? Ub : Ua)[r] = aw[r];
-      // d act / d pre-activation from the activation itself (already computed for dW): LeakyReLU keeps the sign and a
-      // dropped element is exactly 0, so u > 0 -> inv, u < 0 -> slope * inv, u == 0 -> dropped (or a pre-activation of
-      // exactly 0, a null set) -> 0. Saves the second dropout hash and the per-element mask decode of the generic form.
-      float uu[8], yy[8];
-      unpack8(a8, uu);
+      // d act / d pre-activation: the sign of the forward's own fma (the one deferred_act8 just evaluated), times the
+      // dropout mask of that same evaluation (no second hash). A pre-activation of exactly 0 takes the slope branch,
+      // as in every other backward pass and in kernel 2 below; the sign of the stored bf16 activation cannot tell it
+      // (or a positive value below bf16's smallest subnormal) from a dropped element.
+      float yy[8];
       unpack8h(yraw, yy);
 #pragma unroll
       for (int k = 0; k < 8; ++k) {
         const float d_ = du[k >> 1][2 * grp + (k & 1)];
-        const float fac = uu[k] > 0.f ? inv : (uu[k] < 0.f ? sinv : 0.f);
+        const bool kept = (keep[k >> 1] >> (16 * (k & 1))) & 1u;
+        const float fac = kept ? (fmaf(yy[k], K.sc[k], K.sh[k]) > 0.f ? inv : sinv) : 0.f;
         const float dz = d_ * fac;
         s1[k] += dz;
         s2[k] = fmaf(dz, yy[k], s2[k]);

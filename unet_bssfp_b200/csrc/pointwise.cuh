@@ -151,7 +151,8 @@ struct NormActArgs {
 // rounding); the bf16 form is what a weight gradient pairs with its bf16 gradients.
 __device__ __forceinline__ bf16x8 deferred_act8(const bf16x8& yraw, const float (&sc)[8], const float (&sh)[8],
                                                 float slope, bool slope_le1, bool has_drop, unsigned long long e0,
-                                                uint32_t seed, uint32_t thresh, bf16x8* o16 = nullptr) {
+                                                uint32_t seed, uint32_t thresh, bf16x8* o16 = nullptr,
+                                                uint32_t* keep_words = nullptr) {
   float x[8];
   unpack8h(yraw, x);
 #pragma unroll
@@ -171,6 +172,10 @@ __device__ __forceinline__ bf16x8 deferred_act8(const bf16x8& yraw, const float 
 #pragma unroll
     for (int k = 0; k < 4; ++k) w16[k] = pack_f16x2_sat(x[2 * k], x[2 * k + 1]);
     if (has_drop) apply_maskw(*o16, mw);
+  }
+  if (keep_words != nullptr) {   // the dropout mask words (0xFFFF per kept lane), for a backward that needs keep
+#pragma unroll
+    for (int k = 0; k < 4; ++k) keep_words[k] = has_drop ? mw[k] : 0xFFFFFFFFu;
   }
   return o;
 }
@@ -225,8 +230,9 @@ struct DeferredOctet {
     seed = A.drop_seed;
     thresh = A.drop_thresh;
   }
-  __device__ __forceinline__ bf16x8 apply(const bf16x8& yraw, unsigned long long e0, bf16x8* o16 = nullptr) const {
-    return deferred_act8(yraw, sc, sh, slope, slope_le1, has_drop, e0, seed, thresh, o16);
+  __device__ __forceinline__ bf16x8 apply(const bf16x8& yraw, unsigned long long e0, bf16x8* o16 = nullptr,
+                                          uint32_t* keep_words = nullptr) const {
+    return deferred_act8(yraw, sc, sh, slope, slope_le1, has_drop, e0, seed, thresh, o16, keep_words);
   }
 };
 
